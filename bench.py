@@ -7,7 +7,7 @@ degree 10, DEG_ELEV 100: one *eval* = the full constraint vector of one x
 One *step* = one pass over a batch of B such x (the base point and B-1
 finite-difference perturbations of it, which is what SLSQP's Jacobian asks for).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU).  Sharding: the batch of
 perturbed x is split across ranks (each rank evaluates its own B x over all
@@ -31,6 +31,8 @@ if ROOT not in sys.path:
 
 WORKLOAD = dict(N=1024, dim=3, deg=10, elev=100)
 SEED = 20261018
+DUMP_BYTES = 64 * 10 ** 6   # --dump-outputs: at most this much in all
+DUMP_PAIRS = 8192           # --dump-outputs: separation rows of this many pairs (fixed seeded sample)
 
 
 def synthetic_swarm(N, deg, seed=SEED):
@@ -55,6 +57,23 @@ def fd_batch(x, B, seed=1):
     for b, k in enumerate(rng.choice(x.size, size=B - 1, replace=False), start=1):
         X[b, k] += 1.4901161193847656e-08
     return X
+
+
+def dump_outputs(path, pairmin, sep, spd):
+    """Writes what one step of the timed path returned, as float64 .npy files under `path`:
+    pair_min [b, P] (per-pair minima), max_speed [b, N, L] (max-speed rows) and separation
+    [b, DUMP_PAIRS, L] (the separation rows of a fixed, seeded sample of the pairs, in pair order).
+    The full separation block is 2 GB per step, hence the sample; b is the number of leading
+    evaluations of the batch that fit into DUMP_BYTES (all of them at the default batch)."""
+    import torch
+    P, L = sep.shape[1], sep.shape[2]
+    idx = np.sort(np.random.default_rng(SEED).choice(P, size=min(P, DUMP_PAIRS), replace=False))
+    b = min(sep.shape[0], DUMP_BYTES // (8 * (pairmin.shape[1] + spd.shape[1] * spd.shape[2] + idx.size * L)))
+    arrays = {"pair_min": pairmin[:b], "max_speed": spd[:b],
+              "separation": sep[:b].index_select(1, torch.as_tensor(idx, device=sep.device))}
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 # --------------------------------------------------------------------------
@@ -476,6 +495,9 @@ def run_ours(opts):
             dist.all_gather_into_tensor(ref, mine)
         torch.cuda.synchronize()
         assert torch.equal(ref, gathered), "gathered per-pair minima differ from the NCCL all-gather"
+    if opts.dump_outputs and rank == 0:
+        # the last timed step's results, before anything below reuses its buffers (rank 0's share)
+        dump_outputs(opts.dump_outputs, gathered, last_sep, out_spds[(step_no[0] - 1) % nlanes])
 
     # dominant kernel alone (pair kernel over this rank's pairs), CUDA events on its stream
     cpts, tf = eng.assemble(d_x, E)
@@ -959,7 +981,14 @@ def main():
     ap.add_argument("--no-slsqp", action="store_true", help="skip the slsqp_c2 / slsqp_c3 keys")
     ap.add_argument("--slsqp-full", action="store_true",
                     help="run every SLSQP arm of C3 to convergence (the host arm takes minutes)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps write what the last one computed to DIR/<name>.npy (float64, at most "
+                         "64 MB: per-pair minima, max-speed rows, separation rows of a fixed seeded sample of pairs)")
     opts = ap.parse_args()
+    if opts.steps < 1:
+        ap.error("--steps must be at least 1")
+    if opts.dump_outputs and (opts.impl != "ours" or opts.workload != "c4"):
+        ap.error("--dump-outputs applies to the default workload (--impl ours --workload c4)")
     if opts.batch <= 0:
         opts.batch = 32 if opts.scaling == "strong" else 4
     if opts.impl == "reference":

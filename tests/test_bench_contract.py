@@ -66,6 +66,45 @@ def test_both_arms_share_one_config_dict():
     assert d["config"] == cfg
 
 
+def test_dump_outputs_layout_and_budget(tmp_path, monkeypatch):
+    """--dump-outputs: float64 arrays; the separation rows of the same seeded pair sample on every
+    call, in pair order; whole leading evaluations of the batch within the size budget."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    B, P, N, L = 3, 20000, 50, 7
+    pm = torch.randn((B, P), dtype=torch.float64)
+    spd = torch.randn((B, N, L), dtype=torch.float64)
+    sep = torch.arange(P, dtype=torch.float64)[None, :, None] + torch.zeros((B, 1, L), dtype=torch.float64)
+    sep[1] += 0.5
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), pm, sep, spd)
+    out = {f: np.load(str(tmp_path / "a" / f)) for f in os.listdir(str(tmp_path / "a"))}
+    assert set(out) == {"pair_min.npy", "max_speed.npy", "separation.npy"}
+    assert all(a.dtype == np.float64 for a in out.values())
+    assert sum(a.nbytes for a in out.values()) <= bench.DUMP_BYTES
+    assert np.array_equal(out["pair_min.npy"], pm.numpy()) and np.array_equal(out["max_speed.npy"], spd.numpy())
+    s = out["separation.npy"]
+    assert s.shape == (B, bench.DUMP_PAIRS, L)
+    pairs = s[0, :, 0]
+    assert np.all(np.diff(pairs) > 0) and pairs[0] >= 0 and pairs[-1] < P
+    assert np.array_equal(s[1], s[0] + 0.5) and np.array_equal(s[2], s[0])
+    for f, a in out.items():
+        assert np.array_equal(np.load(str(tmp_path / "b" / f)), a)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2 * 8 * (P + N * L + bench.DUMP_PAIRS * L))
+    bench.dump_outputs(str(tmp_path / "c"), pm, sep, spd)
+    assert np.load(str(tmp_path / "c" / "separation.npy")).shape[0] == 2
+    assert np.array_equal(np.load(str(tmp_path / "c" / "pair_min.npy")), pm[:2].numpy())
+
+
+def test_bench_rejects_unsupported_arguments(tmp_path):
+    for argv in (("--steps", "0"), ("--impl", "reference", "--dump-outputs", str(tmp_path / "d")),
+                 ("--workload", "c5", "--dump-outputs", str(tmp_path / "d"))):
+        r = _run(*argv, timeout=60)
+        assert r.returncode != 0 and "usage" in r.stderr
+    assert not os.path.exists(str(tmp_path / "d"))
+
+
 def test_python_reference_leg_when_staged():
     """cpu_baseline_python times the unmodified reference from baseline/_ref (staged by
     __graft_entry__.build() where /root/reference exists); absent copy -> None."""
