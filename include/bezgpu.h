@@ -46,7 +46,8 @@ extern "C" {
  *                                                         variant for L <= 128, column-tiled variant above;
  *                                                         other shapes run the DFMA kernels)
  *   closed-form Jacobian kernels                          n <= BEZ_MAX_DEGREE_JAC  = 12
- *   angular rate                                          n + elev <= 250 (tensor path <= 127) */
+ *   angular rate                                          n + elev <= 250 (tensor path and closed-form
+ *                                                         Jacobian <= 127) */
 #define BEZ_MAX_DEGREE      16
 #define BEZ_MAX_DEGREE_MMA  15
 #define BEZ_MAX_DEGREE_JAC  12
@@ -233,6 +234,29 @@ int bez_fd_quotient(const double *d_F, const double *d_dx, int nvar, int64_t m,
 /* count independent sweeps: d_F [count][nvar+1][m], d_dx [count][nvar], d_JT [count][nvar][m] */
 int bez_fd_quotient_batched(const double *d_F, const double *d_dx, int64_t count, int nvar,
                             int64_t m, double *d_JT, void *stream);
+
+/* Closed-form 2-point quotient of the angular-rate block (bez_angrate_sq with alpha, any beta):
+ * the block is a control-point-wise ratio QQ / SS of two Bernstein squares of bilinear forms in the
+ * control points, and P(a', a') - P(a, a) = P(a' - a, a' + a) (P = Bernstein product) gives every
+ * difference without cancellation (DESIGN section 3.3).  Matches the exactly rounded quotient, and
+ * writes only the rows of the vehicle a control-point variable moves.  n + elev <= 127
+ * (BEZ_EUNSUPPORTED above: bez_fd_quotient covers those shapes).
+ *   d_cpts  [B][N][row_stride]  base points (vehicles 0..numVeh-1 are used);  d_tf [B]
+ *   nvar    numVeh*2*ncols (+ 1 with kdir >= 0); variables in x's order (vehicle, dimension,
+ *           free column; control point = column + offset), then tf
+ *   d_dx    [B][nvar] SciPy's divisors
+ *   d_dir   [N][row_stride] d(control points)/d tf, or NULL (tf moves no control point)
+ *   kdir    nvar-1 for time-optimal models (tf also scales the derivatives), else -1
+ *   dense = 1: d_out is J^T [B][nvar][ld], zero-filled here, ld >= numVeh*(4m+1)
+ *   dense = 0: [B][numVeh*2*ncols + (kdir >= 0 ? numVeh : 0)][4m+1]: one row per control-point
+ *              variable in x's order, then one tf row per vehicle
+ *   d_scratch bez_jac_angrate_scratch_doubles(B, numVeh, n, elev) doubles:
+ *              B*numVeh*(128*U + 432), U = ceil((n+elev+1)/8); 0 for unsupported shapes */
+size_t bez_jac_angrate_scratch_doubles(int B, int numVeh, int n, int elev);
+int bez_jac_angrate_sq(const bez_angrate_tables *tables, const double *d_cpts, const double *d_tf,
+                       int B, int N, int row_stride, int numVeh, int ncols, int offset, int nvar,
+                       const double *d_dx, const double *d_dir, int kdir, double alpha, int dense,
+                       double *d_scratch, double *d_out, int64_t ld, void *stream);
 
 /* ---- single-curve algebra behind the bezier.Bezier methods, batched over
  * independent rows/curves; tables are DEVICE arrays the caller built on the host

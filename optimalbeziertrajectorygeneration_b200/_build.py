@@ -34,6 +34,7 @@ UNITS = [
     ("constraints_mma_speed_b.cu", []),
     ("jacobian.cu", []),
     ("angrate.cu", []),
+    ("angrate_jac.cu", []),
     ("curveops.cu", []),
     ("geometry.cu", ["-fmad=false"]),
 ]

@@ -82,15 +82,25 @@ class ProblemBatch:
 
     def sweep(self, X, elev=None, blocks=("sep", "maxspeed", "angrate")):
         """One finite-difference sweep of every problem: returns {block: (f0 [M, m], JT [M, nvar, m])}
-        on the device, JT[p, k] = (f(x_p + h_k e_k) - f(x_p)) / dx_k (SciPy's 2-point formula)."""
+        on the device, JT[p, k] = (f(x_p + h_k e_k) - f(x_p)) / dx_k (SciPy's 2-point formula).
+        "angrate_closed": the angular-rate block with the closed-form quotient
+        (ConstraintEngine.jac_angrate_closed): values at the M base points only, one Jacobian launch."""
+        literal = tuple(b for b in blocks if b != "angrate_closed")
         Xp, dx = self.fd_points(X)
-        nv1 = self.nvar + 1
-        F = self.evaluate(Xp.view(self.M * nv1, self.nvar), nv1, elev, blocks)
         out = {}
-        for name, f in F.items():
-            mb = int(f.shape[1])
-            JT = torch.empty((self.M, self.nvar, mb), dtype=F64, device=f.device)
-            _capi.call("bez_fd_quotient_batched", _engine._ptr(f), _engine._ptr(dx), self.M, self.nvar, mb,
-                       _engine._ptr(JT), _engine._stream())
-            out[name] = (f.view(self.M, nv1, mb)[:, 0], JT)
+        if literal:
+            nv1 = self.nvar + 1
+            F = self.evaluate(Xp.view(self.M * nv1, self.nvar), nv1, elev, literal)
+            for name, f in F.items():
+                mb = int(f.shape[1])
+                JT = torch.empty((self.M, self.nvar, mb), dtype=F64, device=f.device)
+                _capi.call("bez_fd_quotient_batched", _engine._ptr(f), _engine._ptr(dx), self.M, self.nvar, mb,
+                           _engine._ptr(JT), _engine._stream())
+                out[name] = (f.view(self.M, nv1, mb)[:, 0], JT)
+        if "angrate_closed" in blocks:
+            E = _opt._deg_elev() if elev is None else int(elev)
+            d_X = Xp[:, 0].contiguous()
+            f0 = self.evaluate(d_X, 1, E, ("angrate",))["angrate"]
+            JT = self.eng.jac_angrate_closed(d_X, E, -1.0, dense=True)
+            out["angrate_closed"] = (f0, JT)
         return out

@@ -539,3 +539,59 @@ class ConstraintEngine:
         JT = torch.empty((self.nvar, m), dtype=F64, device=self.device)
         _capi.call("bez_fd_quotient", _ptr(F), _ptr(d_dx), self.nvar, m, _ptr(JT), self._st())
         return JT
+
+    @staticmethod
+    def _fd_steps_device(d_x, abs_step=1.4901161193847656e-08):
+        """dx of :meth:`fd_steps` for a device tensor (the same IEEE operations)."""
+        h = torch.full_like(d_x, abs_step)
+        dx = (d_x + h) - d_x
+        sign = (d_x >= 0).to(F64) * 2 - 1
+        rel = sign * torch.clamp(d_x.abs(), min=1.0) * np.finfo(np.float64).eps ** 0.5
+        h = torch.where(dx == 0, rel, h)
+        return (d_x + h) - d_x
+
+    @_on_device
+    def jac_angrate_closed(self, x, elev, alpha, dense=True, out=None):
+        """Closed-form '2-point' Jacobian of the angular-rate block (bez_jac_angrate_sq): SciPy's
+        quotient for the row alpha * (squared angular rate) + beta, without evaluating the
+        perturbed points.  ``x`` [nvar] or [B, nvar], host or device.
+        dense: J^T [nvar, numVeh*(4m+1)] ([B, nvar, ...] for 2-D x); else the sweep layout
+        [numVeh*2*ncols + (numVeh if time-optimal), 4m+1] (with a leading B for 2-D x).
+        n + elev > 127 raises BezGpuError (jac_angrate covers those shapes)."""
+        if self.dim != 2:
+            raise ValueError('The input curve must be two dimensional,\n'
+                             'instead it is {} dimensional'.format(self.dim))
+        tabs = AngRateTables.get(self.n, elev, self.dev_index)
+        if isinstance(x, torch.Tensor):
+            batched = x.dim() == 2
+            d_x = x.to(device=self.device, dtype=F64).reshape(-1, self.nvar).contiguous()
+            d_dx = self._fd_steps_device(d_x)
+        else:
+            x = np.asarray(x, dtype=np.float64)
+            batched = x.ndim == 2
+            x2 = np.atleast_2d(x)
+            d_x = self.upload(x2)
+            d_dx = torch.as_tensor(self.fd_steps(x2)[1], device=self.device)
+        B = int(d_x.shape[0])
+        cpts, tf = self.assemble(d_x, elev)
+        dirs = self._direction_rows()
+        kdir = self.nvar - 1 if self.timeopt else -1
+        L4 = 4 * (self.n + int(elev)) + 1
+        if dense:
+            shape = (B, self.nvar, self.numVeh * L4)
+        else:
+            shape = (B, self.numVeh * 2 * self.ncols + (self.numVeh if kdir >= 0 else 0), L4)
+        if out is None:
+            out = torch.empty(shape, dtype=F64, device=self.device)
+        else:
+            self._check(out, shape if batched else shape[1:], "out")
+        nscr = int(_capi.lib.bez_jac_angrate_scratch_doubles(B, self.numVeh, self.n, int(elev)))
+        key = ("jac_angrate_scratch", nscr)
+        scratch = getattr(self, "_scratch", {}).get(key)
+        if scratch is None:
+            scratch = torch.empty(max(nscr, 1), dtype=F64, device=self.device)
+            self._scratch = {key: scratch}                 # one cached buffer per engine
+        _capi.call("bez_jac_angrate_sq", tabs.handle, _ptr(cpts), _ptr(tf), B, self.N, self.row_stride,
+                   self.numVeh, self.ncols, self.offset, self.nvar, _ptr(d_dx), _ptr(dirs), kdir,
+                   float(alpha), int(bool(dense)), _ptr(scratch), _ptr(out), shape[2], self._st())
+        return out if batched else out.view(shape[1:])

@@ -392,6 +392,18 @@ class BezOptimization:
             return eng.download(JT, key="jac:angrate", copy=not self.zero_copy_results).T
         return wrapper
 
+    @property
+    def maxAngularRateConstraints_jac_closed(self):
+        """The same quotient in closed form (ConstraintEngine.jac_angrate_closed): no perturbed
+        points are evaluated, no differencing noise (agrees with the exactly rounded quotient to
+        ~1e-9), and a control-point variable touches only its own vehicle's rows.  n + DEG_ELEV
+        <= 127; the literal closure above covers larger degrees."""
+        def wrapper(x):
+            eng = self._engine(with_obstacles=False)
+            JT = eng.jac_angrate_closed(x, _deg_elev(), -1.0)
+            return eng.download(JT, key="jac:angrate_closed", copy=not self.zero_copy_results).T
+        return wrapper
+
     # ------------------------------------------------------------------
     def generateGuess(self, std=0, seed=None):
         """Initial guess of optimization.py:189-240 (host logic): per vehicle the straight
