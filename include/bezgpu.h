@@ -226,6 +226,32 @@ int bez_jac_speed_sq_elev(const bez_plan *plan, const double *d_cpts, int N, int
                           const double *d_dx, const double *d_dir, int kdir, int dense,
                           double *d_out, int64_t ld, void *stream);
 
+/* The same two Jacobians at B base points at once (problem batches, multi-start points): point b
+ * has its own control points, divisors, tf and output block; the direction rows are shared.
+ *   d_cpts [B][N][S]  base points (bez_assemble_cpts / bez_assemble_cpts_sets)
+ *   d_dx   [B][nvar]  nvar = numVeh*dim*ncols (+ 1 with kdir >= 0)
+ *   kdir   -1, or numVeh*dim*ncols for the tf variable of time-optimal models; d_dir may then be
+ *          NULL: tf moves no control point (its separation rows are zero, its speed rows carry
+ *          only the n/tf factor)
+ *   npairs the leading pairs of the lexicographic list that get rows: at least every pair that
+ *          contains a vehicle (P - nObs(nObs-1)/2, vehicles precede obstacles), at most P
+ *   d_tf   [B] tf of each point (the tf that bez_assemble_cpts returned)
+ *   dense = 1: d_out is J^T [B][nvar][ld], ld >= npairs*L (separation) or numVeh*L (speed);
+ *              entries no item writes (pairs without the variable's vehicle) are zero-filled
+ *   dense = 0: separation [B][numVeh*dim*ncols*(N-1) + (kdir >= 0 ? npairs : 0)][L],
+ *              speed [B][numVeh*dim*ncols + (kdir >= 0 ? numVeh : 0)][L]; ld is ignored
+ * With one vehicle (and npairs = N-1, ld = the block), a point's dense block is its sweep block.
+ * B = 0 is a no-op.  BEZ_EINVAL for NULL pointers, negative sizes, npairs or ld out of range;
+ * BEZ_EUNSUPPORTED above BEZ_MAX_DEGREE_JAC.  Arguments are checked before any CUDA call. */
+int bez_jac_sepsq_elev_batched(const bez_plan *plan, const double *d_cpts, int B, int N,
+                               int numVeh, int ncols, int offset, const double *d_dx,
+                               const double *d_dir, int kdir, int64_t npairs, int dense,
+                               double *d_out, int64_t ld, void *stream);
+int bez_jac_speed_sq_elev_batched(const bez_plan *plan, const double *d_cpts, const double *d_tf,
+                                  int B, int N, int numVeh, int ncols, int offset, double alpha,
+                                  const double *d_dx, const double *d_dir, int kdir, int dense,
+                                  double *d_out, int64_t ld, void *stream);
+
 /* Literal 2-point quotient (scipy/optimize/_numdiff.py:709-711) for constraint
  * blocks without a closed form (angular rate): d_F [nvar+1][m] holds f(x0) in row
  * 0 and f(x0 + h_k e_k) in row k+1; d_JT [nvar][m] = (F[k+1] - F[0]) / dx[k]. */

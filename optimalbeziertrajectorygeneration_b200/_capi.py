@@ -82,6 +82,8 @@ SIGNATURES = {
     "bez_fd_quotient_batched": (I, [P, P, L64, I, L64, P, P]),
     "bez_jac_sepsq_elev": (I, [c_plan_p, P, I, I, I, I, P, P, I, I, P, L64, P]),
     "bez_jac_speed_sq_elev": (I, [c_plan_p, P, I, I, I, I, D, D, P, P, I, I, P, L64, P]),
+    "bez_jac_sepsq_elev_batched": (I, [c_plan_p, P, I, I, I, I, I, P, P, I, L64, I, P, L64, P]),
+    "bez_jac_speed_sq_elev_batched": (I, [c_plan_p, P, P, I, I, I, I, I, D, P, P, I, I, P, L64, P]),
     "bez_jac_angrate_scratch_doubles": (ctypes.c_size_t, [I, I, I, I]),
     "bez_jac_angrate_sq": (I, [c_plan_p, P, P, I, I, I, I, I, I, I, P, P, I, D, I, P, P, L64, P]),
 }

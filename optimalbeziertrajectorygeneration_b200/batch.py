@@ -66,9 +66,13 @@ class ProblemBatch:
         """d_X [M * evals_per_problem, nvar] (device) -> {block: [M * evals_per_problem, m_block]}.
         sep: the npairs_x x-dependent pairs x L; maxspeed: numVeh x L; angrate: numVeh x (4(n+E)+1)."""
         E = _opt._deg_elev() if elev is None else int(elev)
+        cpts, tf = self.eng.assemble(d_X, E, obst_sets=self.d_obst, evals_per_set=int(evals_per_problem))
+        return self._values(cpts, tf, E, blocks)
+
+    def _values(self, cpts, tf, E, blocks):
+        """The blocks of evaluate() at assembled points cpts [Q, N, S], tf [Q]."""
         eng, m = self.eng, self.model
-        Q = int(d_X.shape[0])
-        cpts, tf = eng.assemble(d_X, E, obst_sets=self.d_obst, evals_per_set=int(evals_per_problem))
+        Q = int(cpts.shape[0])
         res = {}
         if "sep" in blocks:
             res["sep"] = eng.separation(cpts, E, m["maxSep"], pair_begin=0, npairs=self.npairs_x).view(Q, -1)
@@ -84,8 +88,12 @@ class ProblemBatch:
         """One finite-difference sweep of every problem: returns {block: (f0 [M, m], JT [M, nvar, m])}
         on the device, JT[p, k] = (f(x_p + h_k e_k) - f(x_p)) / dx_k (SciPy's 2-point formula).
         "angrate_closed": the angular-rate block with the closed-form quotient
-        (ConstraintEngine.jac_angrate_closed): values at the M base points only, one Jacobian launch."""
-        literal = tuple(b for b in blocks if b != "angrate_closed")
+        (ConstraintEngine.jac_angrate_closed): values at the M base points only, one Jacobian launch.
+        "sep_closed", "maxspeed_closed", "minspeed_closed": the separation and speed blocks in closed
+        form (ConstraintEngine.jac_separation_batched / jac_speed_batched), same shapes as the literal
+        blocks; they share one assembly of the M base points and evaluate f0 there only."""
+        closed = tuple(b for b in blocks if b in _CLOSED)
+        literal = tuple(b for b in blocks if b != "angrate_closed" and b not in _CLOSED)
         Xp, dx = self.fd_points(X)
         out = {}
         if literal:
@@ -103,4 +111,20 @@ class ProblemBatch:
             f0 = self.evaluate(d_X, 1, E, ("angrate",))["angrate"]
             JT = self.eng.jac_angrate_closed(d_X, E, -1.0, dense=True)
             out["angrate_closed"] = (f0, JT)
+        if closed:
+            E = _opt._deg_elev() if elev is None else int(elev)
+            eng = self.eng
+            cpts, tf = eng.assemble(Xp[:, 0].contiguous(), E, obst_sets=self.d_obst, evals_per_set=1)
+            f0 = self._values(cpts, tf, E, tuple(_CLOSED[b] for b in closed))
+            base = (cpts, tf, dx)
+            for name in closed:
+                if name == "sep_closed":
+                    JT = eng.jac_separation_batched(None, E, npairs=self.npairs_x, base=base)
+                else:
+                    JT = eng.jac_speed_batched(None, E, -1.0 if name == "maxspeed_closed" else 1.0, base=base)
+                out[name] = (f0[_CLOSED[name]], JT)
         return out
+
+
+# closed-form sweep block -> the literal block it reproduces
+_CLOSED = {"sep_closed": "sep", "maxspeed_closed": "maxspeed", "minspeed_closed": "minspeed"}

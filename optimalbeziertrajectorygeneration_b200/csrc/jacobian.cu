@@ -18,6 +18,13 @@
 //   J_SPEED_DIR  item = vehicle v, tf variable (moves control points and the n/tf factor)
 // Output either in the sweep layout [item][L] or scattered into a dense J^T [nvar][ld]
 // (rows of J^T are contiguous, so stores stay coalesced; the host hands SciPy J^T.T).
+//
+// Batches of B base points (problem batches, multi-start): every mode's items repeat per point b,
+// each with its own control points, divisors, tf and output block; the direction rows are shared.
+// Work is cut into 32-item tiles per point (tile w -> point w / tiles_per_point), so a tile never
+// straddles two points: its rows stay one contiguous run of the point's output block even where the
+// point's direction rows sit between its variable rows and the next point's, and the tensor-path
+// tile store and the partner-row runs of the TMA fetch apply unchanged.
 #include <stdlib.h>
 
 #include "sq_elev_core.cuh"
@@ -34,12 +41,16 @@ struct FullWeights { double w[(N_ + 1) * (N_ + 1)]; };
 
 struct JacArgs {
     int early_store;      // A/B: proxy fence + bulk store right behind each m-tile (BEZGPU_MMA_FLAGS bit 8)
-    const double *cpts;   // [N][S] base point
-    const double *dir;    // [N][S] d y / d x_kdir (DIR modes)
-    const double *dx;     // [nvar]
+    const double *cpts;   // [B][N][S] base points
+    const double *dir;    // [N][S] d y / d x_kdir (DIR modes; shared by all points)
+    const double *dx;     // [B][nvar]
+    const double *tfs;    // [B] tf of each point (SPEED modes), or NULL: the scalar tf
     const double *PQ;     // folded elevation table
     double *out;
-    long long nitems;
+    long long nitems;     // items per point
+    long long tpp;        // 32-item tiles per point
+    long long B;
+    long long cstride, dxstride, ostride;   // doubles between consecutive points' cpts, dx, output
     long long ld;         // dense: row length of J^T
     int N, numVeh, L, Lh, LhPad;
     int ncols, offset;    // free columns per row of x, first free control point
@@ -66,6 +77,16 @@ __device__ __forceinline__ PairVarItem pair_var_item(const JacArgs &A, int dim, 
     return it;
 }
 
+// Tile w of the flattened [B][tpp] tile list: point b, first item t0 of the point, live lanes cnt.
+struct JacTile { long long b, t0; int cnt; };
+__device__ __forceinline__ JacTile jac_tile(const JacArgs &A, long long w) {
+    JacTile t;
+    t.b = A.B == 1 ? 0 : w / A.tpp;
+    t.t0 = (w - t.b * A.tpp) << 5;
+    t.cnt = (int)((A.nitems - t.t0) < 32 ? (A.nitems - t.t0) : 32);
+    return t;
+}
+
 // urow (J_PAIR_VAR only, optional): the partner curve's whole row, already in shared memory.
 // ONEHOT + scratch (J_PAIR_VAR only): 2n+1 doubles of shared memory private to the lane (may alias
 // the urow region of the warp: every lane has read its row before anyone writes).  With it the
@@ -73,7 +94,7 @@ __device__ __forceinline__ PairVarItem pair_var_item(const JacArgs &A, int dim, 
 // bits as the dense double loop (all its other terms add +-0), 22 instead of 242 fp64 instructions.
 template <int N_, int DIM, int JMODE, bool ONEHOT = false>
 __device__ __forceinline__ void jac_stage1(const JacArgs &A, const FullWeights<N_> &FW,
-                                           const DiffWeights<N_> &DW, long long item,
+                                           const DiffWeights<N_> &DW, long long b, long long item,
                                            double (&s)[2 * N_ + 1], long long &ro, const double *urow = nullptr,
                                            double *scratch = nullptr) {
     constexpr int NC = N_ + 1;
@@ -81,6 +102,8 @@ __device__ __forceinline__ void jac_stage1(const JacArgs &A, const FullWeights<N
     constexpr bool DIRMODE = (JMODE == J_PAIR_DIR || JMODE == J_SPEED_DIR);
     constexpr int ND = DIRMODE ? DIM : 1;
     const int dim_ncols = DIM * A.ncols;
+    const double *cpts = A.cpts + b * A.cstride;     // this point's control points and divisors
+    const double *dxs = A.dx + b * A.dxstride;
     double a[ND][NC], dl[ND][NC];
     double dxk;
     int c_hot = 0;              // J_PAIR_VAR: delta = sg_hot * e_{c_hot}
@@ -93,7 +116,7 @@ __device__ __forceinline__ void jac_stage1(const JacArgs &A, const FullWeights<N
         const double sg = v < u ? 1.0 : -1.0;
         c_hot = c;
         sg_hot = sg;
-        const double *pv = A.cpts + (size_t)v * S + d * NC;
+        const double *pv = cpts + (size_t)v * S + d * NC;
         if (urow) {                                 // partner row from shared memory (TMA row fetch)
             const double *pu = urow + d * NC;
 #pragma unroll
@@ -103,7 +126,7 @@ __device__ __forceinline__ void jac_stage1(const JacArgs &A, const FullWeights<N
                 dl[0][k] = (k == c) ? sg : 0.0;
             }
         } else {
-            const double *pu = A.cpts + (size_t)u * S + d * NC;
+            const double *pu = cpts + (size_t)u * S + d * NC;
 #pragma unroll
             for (int k = 0; k < NC; ++k) {
                 const double cv = __ldg(pv + k), cu = __ldg(pu + k);
@@ -111,9 +134,9 @@ __device__ __forceinline__ void jac_stage1(const JacArgs &A, const FullWeights<N
                 dl[0][k] = (k == c) ? sg : 0.0;
             }
         }
-        dxk = __ldg(A.dx + kk);
+        dxk = __ldg(dxs + kk);
         const long long p = bez_pair_row_offset(vi, A.N) + (vj - vi - 1);
-        ro = A.dense ? kk * A.ld + p * A.L : item * (long long)A.L;
+        ro = b * A.ostride + (A.dense ? kk * A.ld + p * A.L : item * (long long)A.L);
     } else if (JMODE == J_PAIR_DIR) {
         int vi, vj;
         bez_pair_decode(item, A.N, vi, vj);
@@ -121,21 +144,21 @@ __device__ __forceinline__ void jac_stage1(const JacArgs &A, const FullWeights<N
         for (int d = 0; d < DIM; ++d)
 #pragma unroll
             for (int k = 0; k < NC; ++k) {
-                a[d][k] = __ldg(A.cpts + (size_t)vi * S + d * NC + k) -
-                          __ldg(A.cpts + (size_t)vj * S + d * NC + k);
+                a[d][k] = __ldg(cpts + (size_t)vi * S + d * NC + k) -
+                          __ldg(cpts + (size_t)vj * S + d * NC + k);
                 dl[d][k] = __ldg(A.dir + (size_t)vi * S + d * NC + k) -
                            __ldg(A.dir + (size_t)vj * S + d * NC + k);
             }
-        dxk = __ldg(A.dx + A.kdir);
-        ro = A.dense ? (long long)A.kdir * A.ld + item * A.L : item * (long long)A.L;
+        dxk = __ldg(dxs + A.kdir);
+        ro = b * A.ostride + (A.dense ? (long long)A.kdir * A.ld + item * A.L : item * (long long)A.L);
     } else if (JMODE == J_SPEED_VAR) {
         const long long kk = item;
         const int v = (int)(kk / dim_ncols);
         const int rem = (int)(kk - (long long)v * dim_ncols);
         const int d = rem / A.ncols;
         const int c = A.offset + (rem - d * A.ncols);
-        const double val = (double)N_ / A.tf;
-        const double *pv = A.cpts + (size_t)v * S + d * NC;
+        const double val = (double)N_ / (A.tfs ? __ldg(A.tfs + b) : A.tf);
+        const double *pv = cpts + (size_t)v * S + d * NC;
         double pt[NC], dd[NC], de[NC];
 #pragma unroll
         for (int k = 0; k < NC; ++k) pt[k] = __ldg(pv + k);
@@ -152,21 +175,22 @@ __device__ __forceinline__ void jac_stage1(const JacArgs &A, const FullWeights<N
             a[0][k] = q;
             dl[0][k] = r;
         }
-        dxk = __ldg(A.dx + kk);
-        ro = A.dense ? kk * A.ld + (long long)v * A.L : item * (long long)A.L;
+        dxk = __ldg(dxs + kk);
+        ro = b * A.ostride + (A.dense ? kk * A.ld + (long long)v * A.L : item * (long long)A.L);
     } else {   // J_SPEED_DIR: tf moves the control points (dir) and the n/tf factor
         const int v = (int)item;
-        dxk = __ldg(A.dx + A.kdir);
-        const double val = (double)N_ / A.tf;
-        const double valp = (double)N_ / (A.tf + dxk);
-        const double gam = -(double)N_ / (A.tf * (A.tf + dxk));     // (valp - val) / dx
+        dxk = __ldg(dxs + A.kdir);
+        const double tf = A.tfs ? __ldg(A.tfs + b) : A.tf;
+        const double val = (double)N_ / tf;
+        const double valp = (double)N_ / (tf + dxk);
+        const double gam = -(double)N_ / (tf * (tf + dxk));         // (valp - val) / dx
 #pragma unroll
         for (int d = 0; d < DIM; ++d) {
             double pt[NC], pd[NC], dd[NC], de[NC];
 #pragma unroll
             for (int k = 0; k < NC; ++k) {
-                pt[k] = __ldg(A.cpts + (size_t)v * S + d * NC + k);
-                pd[k] = __ldg(A.dir + (size_t)v * S + d * NC + k);
+                pt[k] = __ldg(cpts + (size_t)v * S + d * NC + k);
+                pd[k] = A.dir ? __ldg(A.dir + (size_t)v * S + d * NC + k) : 0.0;   // NULL: tf moves no point
             }
 #pragma unroll
             for (int k = 0; k < N_; ++k) {
@@ -182,7 +206,7 @@ __device__ __forceinline__ void jac_stage1(const JacArgs &A, const FullWeights<N
                 dl[d][k] = r;
             }
         }
-        ro = A.dense ? (long long)A.kdir * A.ld + (long long)v * A.L : item * (long long)A.L;
+        ro = b * A.ostride + (A.dense ? (long long)A.kdir * A.ld + (long long)v * A.L : item * (long long)A.L);
     }
 
     if (ONEHOT && JMODE == J_PAIR_VAR) {
@@ -231,19 +255,19 @@ jac_sq_elev_kernel(const JacArgs A, const FullWeights<N_> FW, const DiffWeights<
     for (int i = threadIdx.x; i < NT * A.LhPad; i += kThreads) tab[i] = __ldg(A.PQ + i);
     __syncthreads();
 
-    const long long nwt = (A.nitems + 31) >> 5;
+    const long long nwt = A.B * A.tpp;
     const long long gwarp = (long long)blockIdx.x * kWarps + warp;
     const long long nwarps = (long long)gridDim.x * kWarps;
     const int ngroups = (A.LhPad / 32 + CPL - 1) / CPL;
 
     for (long long wt = gwarp; wt < nwt; wt += nwarps) {
-        const long long t0 = wt << 5;
-        const int cnt = (int)((A.nitems - t0) < 32 ? (A.nitems - t0) : 32);
+        const JacTile T = jac_tile(A, wt);
+        const int cnt = T.cnt;
         {
-            const long long item = t0 + (lane < cnt ? lane : cnt - 1);
+            const long long item = T.t0 + (lane < cnt ? lane : cnt - 1);
             double s[2 * N_ + 1];
             long long ro;
-            jac_stage1<N_, DIM, JMODE>(A, FW, DW, item, s, ro);
+            jac_stage1<N_, DIM, JMODE>(A, FW, DW, T.b, item, s, ro);
             rowoff[lane] = ro;
             double2 *row = rows + (size_t)lane * RS;
 #pragma unroll
@@ -283,18 +307,20 @@ jac_sq_elev_mma_kernel(const JacArgs A, const FullWeights<N_> FW, const DiffWeig
     MinSinks no_sinks;
     memset(&no_sinks, 0, sizeof(no_sinks));
     __syncwarp();
-    const long long nwt = (A.nitems + 31) >> 5;
+    const long long nwt = A.B * A.tpp;
     const long long gwarp = (long long)blockIdx.x * kWarps + warp;
     const long long nwarps = (long long)gridDim.x * kWarps;
-    const bool base_aligned = (reinterpret_cast<uintptr_t>(A.out) & 15u) == 0;
     for (long long wt = gwarp; wt < nwt; wt += nwarps) {
-        const long long t0 = wt << 5;
-        const int cnt = (int)((A.nitems - t0) < 32 ? (A.nitems - t0) : 32);
+        const JacTile T = jac_tile(A, wt);
+        const long long t0 = T.t0;
+        const int cnt = T.cnt;
+        double *pout = A.out + T.b * A.ostride;
+        const bool base_aligned = (reinterpret_cast<uintptr_t>(pout) & 15u) == 0;
         {
             double s[2 * N_ + 1];
             long long ro;
-            jac_stage1<N_, DIM, JMODE, JMODE == J_PAIR_VAR>(A, FW, DW, t0 + (lane < cnt ? lane : cnt - 1), s, ro, nullptr,
-                                                            rows + lane * kRowStride);
+            jac_stage1<N_, DIM, JMODE, JMODE == J_PAIR_VAR>(A, FW, DW, T.b, t0 + (lane < cnt ? lane : cnt - 1), s, ro,
+                                                            nullptr, rows + lane * kRowStride);
             double *row = rows + lane * kRowStride;
 #pragma unroll
             for (int j = 0; j < N_; ++j) {
@@ -311,7 +337,7 @@ jac_sq_elev_mma_kernel(const JacArgs A, const FullWeights<N_> FW, const DiffWeig
             }
         }
         __syncwarp();
-        mma_tile<N_, 4, 0, true>(rows, obuf, obuf_s, Bf, A.out + (size_t)t0 * A.L, no_sinks, t0, cnt, A.L, 0.0, lane,
+        mma_tile<N_, 4, 0, true>(rows, obuf, obuf_s, Bf, pout + (size_t)t0 * A.L, no_sinks, t0, cnt, A.L, 0.0, lane,
                                  base_aligned, A.early_store != 0);
         __syncwarp();
     }
@@ -348,7 +374,7 @@ jac_sq_elev_ws_kernel(const JacArgs A, const FullWeights<N_> FW, const DiffWeigh
         }
     }
     __syncthreads();
-    const long long nwt = (A.nitems + 31) >> 5;
+    const long long nwt = A.B * A.tpp;
     const long long ngroups = (long long)gridDim.x * 4, gidx = (long long)blockIdx.x * 4 + group;
     const long long t_begin = gidx * nwt / ngroups;
     const int n = (int)((gidx + 1) * nwt / ngroups - t_begin);
@@ -356,20 +382,21 @@ jac_sq_elev_ws_kernel(const JacArgs A, const FullWeights<N_> FW, const DiffWeigh
         reg_dec<120>();
         for (int k = 0; k < n; ++k) {
             const int s = k % kSlots, use = k / kSlots;
-            const long long t0 = (t_begin + k) << 5;
-            const int cnt = (int)((A.nitems - t0) < 32 ? (A.nitems - t0) : 32);
+            const JacTile T = jac_tile(A, t_begin + k);
+            const int cnt = T.cnt;
+            const double *cpts = A.cpts + T.b * A.cstride;
             double sc[2 * N_ + 1];
             long long ro;
-            const long long item = t0 + (lane < cnt ? lane : cnt - 1);
+            const long long item = T.t0 + (lane < cnt ? lane : cnt - 1);
             double *slot = slots + (size_t)s * kSlotD;
             if (TMAROWS) {
                 // the partner rows of a tile are consecutive rows of the control-point array (one run
                 // per variable, broken once at the owner vehicle): one TMA bulk copy per run
                 const PairVarItem it = pair_var_item(A, DIM, item);
                 // the owner's row and the step length go to L1 while the slot is awaited and the rows fly
-                asm volatile("prefetch.global.L1 [%0];" :: "l"(A.cpts + (size_t)it.v * S_ + it.d * (N_ + 1)));
-                asm volatile("prefetch.global.L1 [%0];" :: "l"(A.cpts + (size_t)it.v * S_ + it.d * (N_ + 1) + N_));
-                asm volatile("prefetch.global.L1 [%0];" :: "l"(A.dx + it.kk));
+                asm volatile("prefetch.global.L1 [%0];" :: "l"(cpts + (size_t)it.v * S_ + it.d * (N_ + 1)));
+                asm volatile("prefetch.global.L1 [%0];" :: "l"(cpts + (size_t)it.v * S_ + it.d * (N_ + 1) + N_));
+                asm volatile("prefetch.global.L1 [%0];" :: "l"(A.dx + T.b * A.dxstride + it.kk));
                 if (use > 0) mbar_wait(empty_b(s), (unsigned)(use - 1) & 1u);
                 const int pu = __shfl_up_sync(0xffffffffu, it.u, 1);
                 const bool start = lane == 0 || it.u != pu + 1;
@@ -381,15 +408,16 @@ jac_sq_elev_ws_kernel(const JacArgs A, const FullWeights<N_> FW, const DiffWeigh
                 if (start) {
                     const unsigned higher = lane == 31 ? 0u : (runs & (0xffffffffu << (lane + 1)));
                     const int end = higher ? __ffs(higher) - 1 : 32;
-                    // a run never leaves the array: rows u .. u + len - 1 <= N - 1 (dead lanes repeat the last item)
-                    bulk_load(slot_s + (unsigned)lane * (S_ * 8u), A.cpts + (size_t)it.u * S_,
+                    // a run never leaves the point's array: rows u .. u + len - 1 <= N - 1 (a tile holds items
+                    // of one point only; dead lanes repeat the last item)
+                    bulk_load(slot_s + (unsigned)lane * (S_ * 8u), cpts + (size_t)it.u * S_,
                               (unsigned)(end - lane) * (S_ * 8u), rows_b(s));
                 }
                 mbar_wait(rows_b(s), (unsigned)use & 1u);
-                jac_stage1<N_, DIM, JMODE, true>(A, FW, DW, item, sc, ro, slot + lane * S_, slot + lane * kRowStride);
+                jac_stage1<N_, DIM, JMODE, true>(A, FW, DW, T.b, item, sc, ro, slot + lane * S_, slot + lane * kRowStride);
                 __syncwarp();
             } else {
-                jac_stage1<N_, DIM, JMODE>(A, FW, DW, item, sc, ro);
+                jac_stage1<N_, DIM, JMODE>(A, FW, DW, T.b, item, sc, ro);
                 if (use > 0) mbar_wait(empty_b(s), (unsigned)(use - 1) & 1u);
             }
             double *row = slot + lane * kRowStride;
@@ -413,19 +441,21 @@ jac_sq_elev_ws_kernel(const JacArgs A, const FullWeights<N_> FW, const DiffWeigh
         const int cidx = warp - kProducers, ci = cidx >> 2;
         double *obuf = stag0 + (size_t)cidx * stag_per;
         const unsigned obuf_s = (unsigned)__cvta_generic_to_shared(obuf);
-        const bool base_aligned = (reinterpret_cast<uintptr_t>(A.out) & 15u) == 0;
         BFrags<N_, 4> Bf;
         load_bfrags<N_, 4>(Bf, A.PQ, A.L, A.LhPad, lane);
         MinSinks no_sinks;
         memset(&no_sinks, 0, sizeof(no_sinks));
         for (int k = ci; k < n; k += 2) {
             const int s = k % kSlots, use = k / kSlots;
-            const long long t0 = (t_begin + k) << 5;
-            const int cnt = (int)((A.nitems - t0) < 32 ? (A.nitems - t0) : 32);
+            const JacTile T = jac_tile(A, t_begin + k);
+            const long long t0 = T.t0;
+            const int cnt = T.cnt;
+            double *pout = A.out + T.b * A.ostride;
+            const bool base_aligned = (reinterpret_cast<uintptr_t>(pout) & 15u) == 0;
             mbar_wait(full_b(s), (unsigned)use & 1u);
             auto release = [&]() { mbar_arrive(empty_b(s)); };
             mma_tile<N_, 4, 0, true, decltype(release)>(slots + (size_t)s * kSlotD, obuf, obuf_s, Bf,
-                                                        A.out + (size_t)t0 * A.L, no_sinks, t0, cnt, A.L, 0.0, lane,
+                                                        pout + (size_t)t0 * A.L, no_sinks, t0, cnt, A.L, 0.0, lane,
                                                         base_aligned, false, release);
             __syncwarp();
         }
@@ -448,7 +478,7 @@ int launch_jac_ws(const bez_plan *plan, const JacArgs &A, cudaStream_t st) {
     auto kern = jac_sq_elev_ws_kernel<N_, DIM, JMODE>;
     int sms = 148, per_sm = 1;
     if (int rc = bez_kernel_config((const void *)kern, bezws::kWsThreads, shmem, &sms, &per_sm)) return rc;
-    const long long nwt = (A.nitems + 31) / 32;
+    const long long nwt = A.B * A.tpp;
     long long grid = sms;
     if (grid > (nwt + 7) / 8) grid = (nwt + 7) / 8;
     if (grid < 1) return BEZ_OK;
@@ -475,7 +505,7 @@ int launch_jac_mma(const bez_plan *plan, const JacArgs &A, cudaStream_t st) {
     auto kern = jac_sq_elev_mma_kernel<N_, DIM, JMODE>;
     int sms = 148, per_sm = 1;
     if (int rc = bez_kernel_config((const void *)kern, kThreads, shmem, &sms, &per_sm)) return rc;
-    const long long nwt = (A.nitems + 31) / 32;
+    const long long nwt = A.B * A.tpp;
     long long grid = (long long)sms * per_sm;
     const long long need = (nwt + kWarps - 1) / kWarps;
     if (grid > need) grid = need;
@@ -501,7 +531,7 @@ int launch_jac(const bez_plan *plan, const JacArgs &A, cudaStream_t st) {
     auto kern = jac_sq_elev_kernel<N_, DIM, JMODE>;
     int sms = 148, per_sm = 1;
     if (int rc = bez_kernel_config((const void *)kern, kThreads, shmem, &sms, &per_sm)) return rc;
-    const long long nwt = (A.nitems + 31) / 32;
+    const long long nwt = A.B * A.tpp;
     long long grid = (long long)sms * per_sm;
     const long long need = (nwt + kWarps - 1) / kWarps;
     if (grid > need) grid = need;
@@ -553,6 +583,7 @@ int fill_common(const bez_plan *plan, JacArgs &A, const double *d_cpts, const do
     A.cpts = d_cpts; A.dir = d_dir; A.dx = d_dx; A.PQ = plan->d_PQ; A.out = d_out;
     A.ld = ld; A.N = N; A.numVeh = numVeh; A.L = plan->L; A.Lh = plan->Lh; A.LhPad = plan->LhPad;
     A.ncols = ncols; A.offset = offset; A.kdir = kdir; A.dense = dense; A.tf = 1.0; A.scale = 1.0;
+    A.tfs = nullptr; A.B = 1; A.cstride = A.dxstride = A.ostride = 0; A.nitems = A.tpp = 0;
     A.early_store = (bez_sq_elev_mma_flags() & kFlagEarlyFence) ? 1 : 0;
     return BEZ_OK;
 }
@@ -607,6 +638,125 @@ extern "C" int bez_fd_quotient(const double *d_F, const double *d_dx, int nvar, 
     return BEZ_OK;
 }
 
+namespace {
+
+// Zero `len` doubles at out + b * stride + off for every point b (rows no item writes).
+__global__ void zero_rows_kernel(double *__restrict__ out, long long B, long long stride, long long off,
+                                 long long len) {
+    const long long total = B * len;
+    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
+         idx += (long long)gridDim.x * blockDim.x) {
+        const long long b = idx / len;
+        out[b * stride + off + (idx - b * len)] = 0.0;
+    }
+}
+
+int zero_rows(double *out, long long B, long long stride, long long off, long long len, cudaStream_t st) {
+    if (B == 0 || len == 0) return BEZ_OK;
+    if (stride == len && off == 0) {
+        BEZ_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * (size_t)(B * len), st));
+        return BEZ_OK;
+    }
+    long long blocks = (B * len + 255) / 256;
+    if (blocks > 148 * 32) blocks = 148 * 32;
+    zero_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(out, B, stride, off, len);
+    BEZ_CUDA(cudaGetLastError());
+    return BEZ_OK;
+}
+
+// Shared body of the single-point and batched separation Jacobians.  With one vehicle, the
+// leading N-1 pairs and ld = (N-1)*L, item (kk, uu) of the dense J^T lands at kk*ld + uu*L and
+// the tf rows at kdir*ld: a point's dense block is its sweep block byte for byte, nothing is left
+// to zero, and the dense request runs as a sweep (on the tensor path where L allows).  The
+// single-point entry keeps its kernel choice (dense_as_sweep = false) so its results stay those
+// of the dense kernel.  kdir >= 0 with d_dir == NULL: tf moves no control point, its rows are 0.
+int jac_sep_impl(const bez_plan *plan, const double *d_cpts, long long B, int N, int numVeh, int ncols,
+                 int offset, const double *d_dx, const double *d_dir, int kdir, long long npairs, int dense,
+                 double *d_out, int64_t ld, bool dense_as_sweep, cudaStream_t st) {
+    const long long L = plan->L;
+    const long long nvarN = (long long)numVeh * plan->dim * ncols;
+    const long long nvar = nvarN + (kdir >= 0 ? 1 : 0);
+    const long long S = (plan->dim * (plan->n + 1) + 1) / 2 * 2;
+    const long long ndir = kdir >= 0 ? npairs : 0;
+    JacArgs A;
+    fill_common(plan, A, d_cpts, d_dir, d_dx, N, numVeh, ncols, offset, kdir, dense, d_out, ld);
+    A.scale = 0.5 * plan->dim;
+    A.B = B;
+    A.cstride = (long long)N * S;
+    A.dxstride = nvar;
+    if (dense && dense_as_sweep && numVeh == 1 && npairs == N - 1 && ld == npairs * L) A.dense = 0;
+    A.ostride = A.dense ? nvar * ld : (nvarN * (N - 1) + ndir) * L;
+    if (A.dense && (numVeh > 1 || npairs > N - 1 || ld > npairs * L)) {
+        // rows of pairs without the variable's vehicle are never written
+        BEZ_CUDA(cudaMemsetAsync(d_out, 0, sizeof(double) * (size_t)(B * nvar * ld), st));
+    } else if (kdir >= 0 && !d_dir) {
+        // the tf rows: J^T row kdir (dense) or the trailing npairs rows (sweep)
+        const long long off = A.dense ? (long long)kdir * ld : nvarN * (N - 1) * L;
+        if (int rc = zero_rows(d_out, B, A.ostride, off, A.dense ? ld : ndir * L, st)) return rc;
+    }
+    A.nitems = nvarN * (N - 1);
+    A.tpp = (A.nitems + 31) / 32;
+    if (A.nitems > 0) {
+        int rc = jdispatch<J_PAIR_VAR>(plan, A, st);
+        if (rc != BEZ_OK) return rc;
+    }
+    if (kdir >= 0 && d_dir && npairs > 0) {
+        if (!A.dense) A.out = d_out + (size_t)A.nitems * L;
+        A.nitems = npairs;
+        A.tpp = (A.nitems + 31) / 32;
+        return jdispatch<J_PAIR_DIR>(plan, A, st);
+    }
+    return BEZ_OK;
+}
+
+// Shared body of the speed Jacobians; d_tf [B] or NULL (the scalar tf).  kdir >= 0 with
+// d_dir == NULL: tf moves no control point, only the n/tf factor.
+int jac_speed_impl(const bez_plan *plan, const double *d_cpts, const double *d_tf, double tf, long long B,
+                   int N, int numVeh, int ncols, int offset, double alpha, const double *d_dx, const double *d_dir,
+                   int kdir, int dense, double *d_out, int64_t ld, bool dense_as_sweep, cudaStream_t st) {
+    const long long L = plan->L;
+    const long long nvarN = (long long)numVeh * plan->dim * ncols;
+    const long long nvar = nvarN + (kdir >= 0 ? 1 : 0);
+    const long long S = (plan->dim * (plan->n + 1) + 1) / 2 * 2;
+    JacArgs A;
+    fill_common(plan, A, d_cpts, d_dir, d_dx, N, numVeh, ncols, offset, kdir, dense, d_out, ld);
+    A.scale = alpha * 0.5 * plan->dim;
+    A.tf = tf;
+    A.tfs = d_tf;
+    A.B = B;
+    A.cstride = (long long)N * S;
+    A.dxstride = nvar;
+    // one vehicle with ld = L: J^T row kk is the sweep row of item kk, the tf row that of vehicle 0
+    if (dense && dense_as_sweep && numVeh == 1 && ld == L) A.dense = 0;
+    A.ostride = A.dense ? nvar * ld : (nvarN + (kdir >= 0 ? numVeh : 0)) * L;
+    if (A.dense && (numVeh > 1 || ld > (long long)numVeh * L))
+        BEZ_CUDA(cudaMemsetAsync(d_out, 0, sizeof(double) * (size_t)(B * nvar * ld), st));
+    A.nitems = nvarN;
+    A.tpp = (A.nitems + 31) / 32;
+    if (A.nitems > 0) {
+        int rc = jdispatch<J_SPEED_VAR>(plan, A, st);
+        if (rc != BEZ_OK) return rc;
+    }
+    if (kdir >= 0) {
+        if (!A.dense) A.out = d_out + (size_t)A.nitems * L;
+        A.nitems = numVeh;
+        A.tpp = (A.nitems + 31) / 32;
+        return jdispatch<J_SPEED_DIR>(plan, A, st);
+    }
+    return BEZ_OK;
+}
+
+int jac_degree_supported(const bez_plan *plan) {
+    if (plan->n < 1 || plan->n > BEZ_MAX_DEGREE_JAC || plan->dim < 1 || plan->dim > 3) {
+        bez_set_error("degree %d, dimension %d: the Jacobian kernels cover n <= %d, dim <= 3", plan->n, plan->dim,
+                      BEZ_MAX_DEGREE_JAC);
+        return BEZ_EUNSUPPORTED;
+    }
+    return BEZ_OK;
+}
+
+}  // namespace
+
 extern "C" int bez_jac_sepsq_elev(const bez_plan *plan, const double *d_cpts, int N, int numVeh,
                                   int ncols, int offset, const double *d_dx, const double *d_dir,
                                   int kdir, int dense, double *d_out, int64_t ld, void *stream) {
@@ -614,28 +764,10 @@ extern "C" int bez_jac_sepsq_elev(const bez_plan *plan, const double *d_cpts, in
     BEZ_REQUIRE(N >= 2 && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0, "bad sizes");
     BEZ_REQUIRE(kdir < 0 || d_dir, "direction rows are NULL");
     const long long P = (long long)N * (N - 1) / 2;
-    const long long nvarN = (long long)numVeh * plan->dim * ncols;
     BEZ_REQUIRE(!dense || ld >= P * plan->L, "ld smaller than the constraint block");
     BEZ_ON_DEVICE(plan->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    JacArgs A;
-    fill_common(plan, A, d_cpts, d_dir, d_dx, N, numVeh, ncols, offset, kdir, dense, d_out, ld);
-    A.scale = 0.5 * plan->dim;
-    if (dense) {
-        const long long nvar = nvarN + (kdir >= 0 ? 1 : 0);
-        BEZ_CUDA(cudaMemsetAsync(d_out, 0, sizeof(double) * (size_t)nvar * (size_t)ld, st));
-    }
-    A.nitems = nvarN * (N - 1);
-    if (A.nitems > 0) {
-        int rc = jdispatch<J_PAIR_VAR>(plan, A, st);
-        if (rc != BEZ_OK) return rc;
-    }
-    if (kdir >= 0) {
-        if (!dense) A.out = d_out + (size_t)A.nitems * plan->L;
-        A.nitems = P;
-        return jdispatch<J_PAIR_DIR>(plan, A, st);
-    }
-    return BEZ_OK;
+    return jac_sep_impl(plan, d_cpts, 1, N, numVeh, ncols, offset, d_dx, d_dir, kdir, P, dense, d_out, ld, false,
+                        (cudaStream_t)stream);
 }
 
 extern "C" int bez_jac_speed_sq_elev(const bez_plan *plan, const double *d_cpts, int N, int numVeh,
@@ -645,27 +777,43 @@ extern "C" int bez_jac_speed_sq_elev(const bez_plan *plan, const double *d_cpts,
     BEZ_REQUIRE(plan && d_cpts && d_dx && d_out, "NULL argument");
     BEZ_REQUIRE(N >= 1 && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0, "bad sizes");
     BEZ_REQUIRE(kdir < 0 || d_dir, "direction rows are NULL");
-    const long long nvarN = (long long)numVeh * plan->dim * ncols;
     BEZ_REQUIRE(!dense || ld >= (long long)numVeh * plan->L, "ld smaller than the constraint block");
     BEZ_ON_DEVICE(plan->device);
-    cudaStream_t st = (cudaStream_t)stream;
-    JacArgs A;
-    fill_common(plan, A, d_cpts, d_dir, d_dx, N, numVeh, ncols, offset, kdir, dense, d_out, ld);
-    A.scale = alpha * 0.5 * plan->dim;
-    A.tf = tf;
-    if (dense) {
-        const long long nvar = nvarN + (kdir >= 0 ? 1 : 0);
-        BEZ_CUDA(cudaMemsetAsync(d_out, 0, sizeof(double) * (size_t)nvar * (size_t)ld, st));
-    }
-    A.nitems = nvarN;
-    if (A.nitems > 0) {
-        int rc = jdispatch<J_SPEED_VAR>(plan, A, st);
-        if (rc != BEZ_OK) return rc;
-    }
-    if (kdir >= 0) {
-        if (!dense) A.out = d_out + (size_t)A.nitems * plan->L;
-        A.nitems = numVeh;
-        return jdispatch<J_SPEED_DIR>(plan, A, st);
-    }
-    return BEZ_OK;
+    return jac_speed_impl(plan, d_cpts, nullptr, tf, 1, N, numVeh, ncols, offset, alpha, d_dx, d_dir, kdir, dense,
+                          d_out, ld, false, (cudaStream_t)stream);
+}
+
+extern "C" int bez_jac_sepsq_elev_batched(const bez_plan *plan, const double *d_cpts, int B, int N,
+                                          int numVeh, int ncols, int offset, const double *d_dx,
+                                          const double *d_dir, int kdir, int64_t npairs, int dense,
+                                          double *d_out, int64_t ld, void *stream) {
+    BEZ_REQUIRE(plan && d_cpts && d_dx && d_out, "NULL argument");
+    BEZ_REQUIRE(B >= 0 && N >= 2 && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0, "bad sizes");
+    const long long nvarN = (long long)numVeh * plan->dim * ncols;
+    BEZ_REQUIRE(kdir < 0 || kdir == nvarN, "kdir must be -1 or the index after the control-point variables");
+    const long long P = (long long)N * (N - 1) / 2, nObs = N - numVeh;
+    BEZ_REQUIRE(npairs >= P - nObs * (nObs - 1) / 2 && npairs <= P,
+                "npairs must cover every pair that contains a vehicle and at most all pairs");
+    BEZ_REQUIRE(!dense || ld >= npairs * plan->L, "ld smaller than the constraint block");
+    if (int rc = jac_degree_supported(plan)) return rc;
+    if (B == 0) return BEZ_OK;
+    BEZ_ON_DEVICE(plan->device);
+    return jac_sep_impl(plan, d_cpts, B, N, numVeh, ncols, offset, d_dx, d_dir, kdir, npairs, dense, d_out, ld, true,
+                        (cudaStream_t)stream);
+}
+
+extern "C" int bez_jac_speed_sq_elev_batched(const bez_plan *plan, const double *d_cpts, const double *d_tf,
+                                             int B, int N, int numVeh, int ncols, int offset, double alpha,
+                                             const double *d_dx, const double *d_dir, int kdir, int dense,
+                                             double *d_out, int64_t ld, void *stream) {
+    BEZ_REQUIRE(plan && d_cpts && d_tf && d_dx && d_out, "NULL argument");
+    BEZ_REQUIRE(B >= 0 && N >= 1 && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0, "bad sizes");
+    const long long nvarN = (long long)numVeh * plan->dim * ncols;
+    BEZ_REQUIRE(kdir < 0 || kdir == nvarN, "kdir must be -1 or the index after the control-point variables");
+    BEZ_REQUIRE(!dense || ld >= (long long)numVeh * plan->L, "ld smaller than the constraint block");
+    if (int rc = jac_degree_supported(plan)) return rc;
+    if (B == 0) return BEZ_OK;
+    BEZ_ON_DEVICE(plan->device);
+    return jac_speed_impl(plan, d_cpts, d_tf, 1.0, B, N, numVeh, ncols, offset, alpha, d_dx, d_dir, kdir, dense,
+                          d_out, ld, true, (cudaStream_t)stream);
 }

@@ -521,6 +521,82 @@ class ConstraintEngine:
                    ld, self._st())
         return out
 
+    def _batch_points(self, x):
+        """x [B, nvar] (host or device) -> (device x [B, nvar], SciPy's divisors [B, nvar])."""
+        if isinstance(x, torch.Tensor):
+            if x.dim() != 2 or int(x.shape[1]) != self.nvar:
+                raise ValueError("x must be [B, %d]" % self.nvar)
+            d_x = x.to(device=self.device, dtype=F64).contiguous()
+            return d_x, self._fd_steps_device(d_x)
+        x = np.asarray(x, dtype=np.float64)
+        if x.ndim != 2 or x.shape[1] != self.nvar:
+            raise ValueError("x must be [B, %d]" % self.nvar)
+        return self.upload(x), torch.as_tensor(self.fd_steps(x)[1], device=self.device)
+
+    def _batch_out(self, out, shape):
+        if out is None:
+            return torch.empty(shape, dtype=F64, device=self.device)
+        if tuple(out.shape) != shape or out.dtype != F64 or not out.is_contiguous():
+            raise ValueError("out must be a contiguous float64 tensor of shape %r" % (shape,))
+        self._check(out, shape, "out")
+        return out
+
+    @_on_device
+    def jac_separation_batched(self, x, elev, obst_sets=None, npairs=None, dense=True, out=None, base=None):
+        """SciPy's 2-point Jacobian of the separation block at B base points at once
+        (bez_jac_sepsq_elev_batched).  ``x`` [B, nvar], host or device; ``obst_sets``
+        [B, nObs, dim] (device): point b's own obstacles (problem batches); ``npairs``: the
+        leading pairs that get rows (default all; at least every pair with a vehicle).
+        dense: J^T [B, nvar, npairs*L]; else the sweep layout
+        [B, numVeh*dim*ncols*(N-1) + (npairs if time-optimal), L].
+        ``base``: (cpts, tf, dx) of assemble(x) already at hand (ProblemBatch.sweep)."""
+        plan = self.plan(elev)
+        P, L = num_pairs(self.N), plan.L
+        npairs = P if npairs is None else int(npairs)
+        if base is None:
+            d_x, d_dx = self._batch_points(x)
+            cpts, _ = self.assemble(d_x, elev, obst_sets=obst_sets, evals_per_set=1 if obst_sets is not None else 0)
+        else:
+            cpts, _, d_dx = base
+        B = int(cpts.shape[0])
+        kdir = self.nvar - 1 if self.timeopt else -1
+        nvarN = self.numVeh * self.dim * self.ncols
+        if dense:
+            shape = (B, self.nvar, npairs * L)
+        else:
+            shape = (B, nvarN * (self.N - 1) + (npairs if kdir >= 0 else 0), L)
+        out = self._batch_out(out, shape)
+        _capi.call("bez_jac_sepsq_elev_batched", plan.handle, _ptr(cpts), B, self.N, self.numVeh, self.ncols,
+                   self.offset, _ptr(d_dx), _ptr(self._direction_rows()), kdir, npairs, int(bool(dense)), _ptr(out),
+                   npairs * L if dense else 0, self._st())
+        return out
+
+    @_on_device
+    def jac_speed_batched(self, x, elev, alpha, dense=True, out=None, base=None):
+        """SciPy's 2-point Jacobian of the speed block alpha * (squared speed) + beta at B base
+        points at once (bez_jac_speed_sq_elev_batched); tf of each point from assemble.
+        dense: J^T [B, nvar, numVeh*L]; else [B, numVeh*dim*ncols + (numVeh if time-optimal), L].
+        ``base``: (cpts, tf, dx) of assemble(x) already at hand."""
+        plan = self.plan(elev)
+        L = plan.L
+        if base is None:
+            d_x, d_dx = self._batch_points(x)
+            cpts, tf = self.assemble(d_x, elev)
+        else:
+            cpts, tf, d_dx = base
+        B = int(cpts.shape[0])
+        kdir = self.nvar - 1 if self.timeopt else -1
+        nvarN = self.numVeh * self.dim * self.ncols
+        if dense:
+            shape = (B, self.nvar, self.numVeh * L)
+        else:
+            shape = (B, nvarN + (self.numVeh if kdir >= 0 else 0), L)
+        out = self._batch_out(out, shape)
+        _capi.call("bez_jac_speed_sq_elev_batched", plan.handle, _ptr(cpts), _ptr(tf), B, int(cpts.shape[1]),
+                   self.numVeh, self.ncols, self.offset, float(alpha), _ptr(d_dx), _ptr(self._direction_rows()),
+                   kdir, int(bool(dense)), _ptr(out), self.numVeh * L if dense else 0, self._st())
+        return out
+
     @_on_device
     def jac_angrate(self, x, elev, alpha, beta):
         """Literal '2-point' FD Jacobian of the angular-rate block: base point and

@@ -475,6 +475,32 @@ class BezOptimization:
         return res
 
     @_on_model_device
+    def jacobian_batch(self, X, which=('sep', 'maxspeed'), elev=None):
+        """The Jacobian counterpart of evaluate_batch: SciPy's 2-point J^T of the named blocks
+        ('sep', 'maxspeed', 'minspeed') at every row of X [B, nvar] (host or device), in closed
+        form and one launch per block; returns device tensors {name: J^T [B, nvar, m_name]}
+        (row b equals the transposed result of the *_jac closure at X[b])."""
+        E = _deg_elev() if elev is None else int(elev)
+        res = {}
+        if 'sep' in which:
+            eng = self._engine(with_obstacles=True)
+            if eng.N <= 1:
+                B = int(X.shape[0]) if isinstance(X, torch.Tensor) else np.atleast_2d(X).shape[0]
+                res['sep'] = torch.empty((B, eng.nvar, 0), dtype=torch.float64, device=eng.device)
+            else:
+                res['sep'] = eng.jac_separation_batched(X, E, dense=True)
+        if 'maxspeed' in which or 'minspeed' in which:
+            eng = self._engine(with_obstacles=False)
+            d_x, d_dx = eng._batch_points(X)
+            cpts, tf = eng.assemble(d_x, E)
+            base = (cpts, tf, d_dx)
+            if 'maxspeed' in which:
+                res['maxspeed'] = eng.jac_speed_batched(None, E, -1.0, base=base)
+            if 'minspeed' in which:
+                res['minspeed'] = eng.jac_speed_batched(None, E, 1.0, base=base)
+        return res
+
+    @_on_model_device
     def evaluate_reduced(self, X, elev=None):
         """Additive API for swarms whose full constraint vector is consumed on the
         device (508 MB per x at N=1024): host X [B, nvar] -> host arrays
