@@ -188,6 +188,9 @@ int bez_speed_sq_elev(const bez_plan *plan, const double *d_cpts, const double *
  *   h_Cm [m+1] = C(m,.)     h_C2m [2m+1] = C(2m,.)
  *   d_out [B][nveh][4m+1] = alpha * (num^2/den^2) + beta   (max rate: alpha=-1, beta=maxAngRate^2)
  *   row_stride = S of the control-point rows (see top of file)
+ * m <= 250 (bez_angrate_tables_create refuses more).  The result does not depend on the spatial
+ * unit: control points x 2^k give bit-identical outputs as long as the Bernstein coefficients of
+ * num^2 and den^2 stay within about 1e+-150 (any m <= 250).
  */
 typedef struct bez_angrate_tables bez_angrate_tables;
 int bez_angrate_tables_create(int n, int elev, int device, const double *h_Tpos,

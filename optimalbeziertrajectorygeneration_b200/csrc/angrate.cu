@@ -15,6 +15,18 @@
 // (bezier.py:1183-1208 at m = 110) nor C(4m,.) is ever formed.  The squares
 // (2 x (2m+1)^2 MACs) use a 4-output register tile with a sliding window so
 // that shared-memory traffic is one load per two DFMAs.
+//
+// Range: coefficient k of a pre-scaled square carries C(4m,k), which runs from 1 at
+// the ends to C(4m,2m) ~ 2^(4m) in the middle -- 2^503 at m = 127, 2^995 at m = 250.
+// angrate_kernel therefore multiplies its degree-2m rows by 2^-s with
+// s = floor(log2 C(4m,2m) / 4) (angrate_v1_shrink), which centres the squares'
+// binomial factors on 1: they span 2^-2s .. 2^(log2 C(4m,2m) - 2s), about 2^+-497 at
+// m = 250.  The factor is exact and cancels in NUM^2 / DEN^2 (the output does not
+// change unless it would leave the fp64 range), and the data's squared numerator and
+// denominator may range over about 2^+-525 (1e+-158) at m = 250; unscaled, the middle
+// coefficients would overflow once they exceed about 7e8.  The m <= 127 kernels keep
+// the unscaled rows: with at most 2^503 in the middle the data keeps 2^520 of headroom.
+#include <math.h>
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -33,7 +45,8 @@ struct AngArgs {
     double alpha, beta;
 };
 
-__global__ void __launch_bounds__(kAThreads) angrate_kernel(const AngArgs A) {
+// shrink = 2^-s of angrate_v1_shrink: applied to the degree-2m rows (see the top of the file)
+__global__ void __launch_bounds__(kAThreads) angrate_kernel(const AngArgs A, const double shrink) {
     extern __shared__ __align__(16) double sm[];
     const int m = A.m, n = A.n, m1 = m + 1, L2 = 2 * m + 1;
     double *px = sm, *py = px + m1;
@@ -97,7 +110,7 @@ __global__ void __launch_bounds__(kAThreads) angrate_kernel(const AngArgs A) {
         yD[k] *= c;
     }
     __syncthreads();
-    // degree-2m curves, kept pre-scaled by C(2m,k):
+    // degree-2m curves, kept pre-scaled by C(2m,k) and by the exact power of two 2^-s:
     //   NUM = y''*x' - x''*y'      DEN = x'*x' + y'*y'      (optimization.py:603,605)
     for (int k = tid; k < L2; k += kAThreads) {
         const int ilo = k > m ? k - m : 0, ihi = k < m ? k : m;
@@ -109,8 +122,8 @@ __global__ void __launch_bounds__(kAThreads) angrate_kernel(const AngArgs A) {
             q1 = fma(xD[i], x1, q1);
             q2 = fma(yD[i], y1, q2);
         }
-        NUM[k] = p1 - p2;
-        DEN[k] = q1 + q2;
+        NUM[k] = (p1 - p2) * shrink;
+        DEN[k] = (q1 + q2) * shrink;
     }
     __syncthreads();
     // squares (optimization.py:604,606) and the control-point-wise ratio (:608);
@@ -698,6 +711,13 @@ static WarpPlan2 make_warp_plan2(int m) {
     return W;
 }
 
+// 2^-s, s = floor(log2 C(4m,2m) / 4): the scale of angrate_kernel's degree-2m rows
+static double angrate_v1_shrink(int m) {
+    double l = 0.0;
+    for (int k = 1; k <= 2 * m; ++k) l += log2((double)(2 * m + k) / k);    // log2 C(4m,2m)
+    return ldexp(1.0, -(int)(l / 4));
+}
+
 static WarpPlan make_warp_plan(int m) {
     WarpPlan W;
     const int m1 = m + 1, L2 = 2 * m + 1;
@@ -731,8 +751,12 @@ extern "C" int bez_angrate_tables_create(int n, int elev, int device, const doub
     BEZ_REQUIRE(h_Tpos && h_elev1m && h_Cm && h_C2m, "tables are NULL");
     BEZ_REQUIRE(n >= 1 && elev >= 0, "bad degree / elevation");
     const int m = n + elev;
+    // m <= 250: the squares' binomial factors C(4m,k) 2^-2s span about 2^+-497 at m = 250 (see the
+    // top of the file), which leaves the data's squared numerator and denominator about 2^+-525;
+    // every extra degree takes 2 bits from both ends
     if (m > 250) {
-        bez_set_error("bez_angrate_tables_create: n+elev = %d > 250 (C(2m,m)^2 would overflow fp64)", m);
+        bez_set_error("bez_angrate_tables_create: n+elev = %d > 250 (the binomial factors C(4m,k) of the "
+                      "degree-4m squares would leave the data too little fp64 range)", m);
         return BEZ_EUNSUPPORTED;
     }
     BEZ_ON_DEVICE(device);
@@ -825,7 +849,8 @@ extern "C" int bez_angrate_sq(const bez_angrate_tables *t, const double *d_cpts,
     const size_t shmem = sizeof(double) * ((size_t)8 * (t->m + 1) + 2 * (2 * t->m + 1 + 2 * kPad) + kPad);
     int sms_ = 0, per_sm_ = 0;
     if (int rc = bez_kernel_config((const void *)angrate_kernel, kAThreads, shmem, &sms_, &per_sm_)) return rc;
-    angrate_kernel<<<(unsigned)((long long)B * nveh), kAThreads, shmem, (cudaStream_t)stream>>>(A);
+    angrate_kernel<<<(unsigned)((long long)B * nveh), kAThreads, shmem, (cudaStream_t)stream>>>(
+        A, angrate_v1_shrink(t->m));
     BEZ_CUDA(cudaGetLastError());
     return BEZ_OK;
 }
