@@ -218,6 +218,8 @@ int bez_angrate_sq(const bez_angrate_tables *tables, const double *d_cpts, const
  *   dense = 0: sweep layout, [numVeh*dim*ncols][N-1][L] (partner curves in
  *              ascending order, the vehicle itself skipped) followed, when
  *              kdir >= 0, by [P][L] for the kdir column.
+ * These two are the B = 1 case of the batched entries below (all P pairs; the scalar tf for the
+ * speed rows): the same argument checks and the same kernel choice.
  */
 int bez_jac_sepsq_elev(const bez_plan *plan, const double *d_cpts, int N, int numVeh,
                        int ncols, int offset, const double *d_dx, const double *d_dir,
@@ -243,9 +245,11 @@ int bez_jac_speed_sq_elev(const bez_plan *plan, const double *d_cpts, int N, int
  *              entries no item writes (pairs without the variable's vehicle) are zero-filled
  *   dense = 0: separation [B][numVeh*dim*ncols*(N-1) + (kdir >= 0 ? npairs : 0)][L],
  *              speed [B][numVeh*dim*ncols + (kdir >= 0 ? numVeh : 0)][L]; ld is ignored
- * With one vehicle (and npairs = N-1, ld = the block), a point's dense block is its sweep block.
- * B = 0 is a no-op.  BEZ_EINVAL for NULL pointers, negative sizes, npairs or ld out of range;
- * BEZ_EUNSUPPORTED above BEZ_MAX_DEGREE_JAC.  Arguments are checked before any CUDA call. */
+ * With one vehicle (and npairs = N-1, ld = the block), a point's dense block is its sweep block,
+ * and a dense request runs as a sweep.
+ * B = 0 is a no-op.  BEZ_EINVAL for NULL pointers, negative sizes, a kdir other than -1 or
+ * numVeh*dim*ncols, npairs or ld out of range; BEZ_EUNSUPPORTED above BEZ_MAX_DEGREE_JAC.
+ * Arguments are checked before any CUDA call. */
 int bez_jac_sepsq_elev_batched(const bez_plan *plan, const double *d_cpts, int B, int N,
                                int numVeh, int ncols, int offset, const double *d_dx,
                                const double *d_dir, int kdir, int64_t npairs, int dense,
@@ -257,7 +261,8 @@ int bez_jac_speed_sq_elev_batched(const bez_plan *plan, const double *d_cpts, co
 
 /* Literal 2-point quotient (scipy/optimize/_numdiff.py:709-711) for constraint
  * blocks without a closed form (angular rate): d_F [nvar+1][m] holds f(x0) in row
- * 0 and f(x0 + h_k e_k) in row k+1; d_JT [nvar][m] = (F[k+1] - F[0]) / dx[k]. */
+ * 0 and f(x0 + h_k e_k) in row k+1; d_JT [nvar][m] = (F[k+1] - F[0]) / dx[k]
+ * (bez_fd_quotient_batched with count = 1). */
 int bez_fd_quotient(const double *d_F, const double *d_dx, int nvar, int64_t m,
                     double *d_JT, void *stream);
 /* count independent sweeps: d_F [count][nvar+1][m], d_dx [count][nvar], d_JT [count][nvar][m] */

@@ -16,11 +16,7 @@ obstacle-obstacle rows of the reference's vector are constants.
 import numpy as np
 import torch
 
-from . import _capi
-from . import engine as _engine
 from . import optimization as _opt
-
-F64 = torch.float64
 
 
 class ProblemBatch:
@@ -50,17 +46,11 @@ class ProblemBatch:
     # ------------------------------------------------------------------
     def fd_points(self, X):
         """host X [M, nvar] -> device (Xp [M, nvar+1, nvar], dx [M, nvar]): the base point and the
-        nvar forward points of every problem, h and dx as SciPy chooses them (engine.fd_steps)."""
-        X = np.ascontiguousarray(np.atleast_2d(np.asarray(X, dtype=np.float64)))
+        nvar forward points of every problem, h and dx as SciPy chooses them (ConstraintEngine.fd_points)."""
+        X = np.atleast_2d(np.asarray(X, dtype=np.float64))
         if X.shape != (self.M, self.nvar):
             raise ValueError("X must be [%d, %d]" % (self.M, self.nvar))
-        h, dx = _engine.ConstraintEngine.fd_steps(X)
-        d_x = torch.as_tensor(X, device=self.eng.device)
-        d_h = torch.as_tensor(h, device=self.eng.device)
-        Xp = d_x[:, None, :].repeat(1, self.nvar + 1, 1)
-        idx = torch.arange(self.nvar, device=self.eng.device)
-        Xp[:, idx + 1, idx] = d_x + d_h
-        return Xp, torch.as_tensor(dx, device=self.eng.device)
+        return self.eng.fd_points(X)
 
     def evaluate(self, d_X, evals_per_problem, elev=None, blocks=("sep", "maxspeed", "angrate")):
         """d_X [M * evals_per_problem, nvar] (device) -> {block: [M * evals_per_problem, m_block]}.
@@ -87,44 +77,36 @@ class ProblemBatch:
     def sweep(self, X, elev=None, blocks=("sep", "maxspeed", "angrate")):
         """One finite-difference sweep of every problem: returns {block: (f0 [M, m], JT [M, nvar, m])}
         on the device, JT[p, k] = (f(x_p + h_k e_k) - f(x_p)) / dx_k (SciPy's 2-point formula).
-        "angrate_closed": the angular-rate block with the closed-form quotient
-        (ConstraintEngine.jac_angrate_closed): values at the M base points only, one Jacobian launch.
-        "sep_closed", "maxspeed_closed", "minspeed_closed": the separation and speed blocks in closed
-        form (ConstraintEngine.jac_separation_batched / jac_speed_batched), same shapes as the literal
-        blocks; they share one assembly of the M base points and evaluate f0 there only."""
+        "sep_closed", "maxspeed_closed", "minspeed_closed", "angrate_closed": the same blocks in closed
+        form (ConstraintEngine.jac_separation / jac_speed / jac_angrate_closed), same shapes as the
+        literal blocks; they share one assembly of the M base points and evaluate f0 there only."""
         closed = tuple(b for b in blocks if b in _CLOSED)
-        literal = tuple(b for b in blocks if b != "angrate_closed" and b not in _CLOSED)
+        literal = tuple(b for b in blocks if b not in _CLOSED)
         Xp, dx = self.fd_points(X)
+        eng = self.eng
         out = {}
         if literal:
             nv1 = self.nvar + 1
             F = self.evaluate(Xp.view(self.M * nv1, self.nvar), nv1, elev, literal)
             for name, f in F.items():
-                mb = int(f.shape[1])
-                JT = torch.empty((self.M, self.nvar, mb), dtype=F64, device=f.device)
-                _capi.call("bez_fd_quotient_batched", _engine._ptr(f), _engine._ptr(dx), self.M, self.nvar, mb,
-                           _engine._ptr(JT), _engine._stream())
-                out[name] = (f.view(self.M, nv1, mb)[:, 0], JT)
-        if "angrate_closed" in blocks:
-            E = _opt._deg_elev() if elev is None else int(elev)
-            d_X = Xp[:, 0].contiguous()
-            f0 = self.evaluate(d_X, 1, E, ("angrate",))["angrate"]
-            JT = self.eng.jac_angrate_closed(d_X, E, -1.0, dense=True)
-            out["angrate_closed"] = (f0, JT)
+                f = f.view(self.M, nv1, -1)
+                out[name] = (f[:, 0], eng.fd_quotient(f, dx))
         if closed:
             E = _opt._deg_elev() if elev is None else int(elev)
-            eng = self.eng
             cpts, tf = eng.assemble(Xp[:, 0].contiguous(), E, obst_sets=self.d_obst, evals_per_set=1)
             f0 = self._values(cpts, tf, E, tuple(_CLOSED[b] for b in closed))
-            base = (cpts, tf, dx)
+            base = (cpts, tf, dx, True)
             for name in closed:
                 if name == "sep_closed":
-                    JT = eng.jac_separation_batched(None, E, npairs=self.npairs_x, base=base)
+                    JT = eng.jac_separation(None, E, npairs=self.npairs_x, base=base)
+                elif name == "angrate_closed":
+                    JT = eng.jac_angrate_closed(None, E, -1.0, base=base)
                 else:
-                    JT = eng.jac_speed_batched(None, E, -1.0 if name == "maxspeed_closed" else 1.0, base=base)
+                    JT = eng.jac_speed(None, E, -1.0 if name == "maxspeed_closed" else 1.0, base=base)
                 out[name] = (f0[_CLOSED[name]], JT)
         return out
 
 
 # closed-form sweep block -> the literal block it reproduces
-_CLOSED = {"sep_closed": "sep", "maxspeed_closed": "maxspeed", "minspeed_closed": "minspeed"}
+_CLOSED = {"sep_closed": "sep", "maxspeed_closed": "maxspeed", "minspeed_closed": "minspeed",
+           "angrate_closed": "angrate"}

@@ -577,31 +577,10 @@ int jdispatch(const bez_plan *plan, const JacArgs &A, cudaStream_t st) {
     return BEZ_EUNSUPPORTED;
 }
 
-int fill_common(const bez_plan *plan, JacArgs &A, const double *d_cpts, const double *d_dir,
-                const double *d_dx, int N, int numVeh, int ncols, int offset, int kdir, int dense,
-                double *d_out, int64_t ld) {
-    A.cpts = d_cpts; A.dir = d_dir; A.dx = d_dx; A.PQ = plan->d_PQ; A.out = d_out;
-    A.ld = ld; A.N = N; A.numVeh = numVeh; A.L = plan->L; A.Lh = plan->Lh; A.LhPad = plan->LhPad;
-    A.ncols = ncols; A.offset = offset; A.kdir = kdir; A.dense = dense; A.tf = 1.0; A.scale = 1.0;
-    A.tfs = nullptr; A.B = 1; A.cstride = A.dxstride = A.ostride = 0; A.nitems = A.tpp = 0;
-    A.early_store = (bez_sq_elev_mma_flags() & kFlagEarlyFence) ? 1 : 0;
-    return BEZ_OK;
-}
-
-// literal 2-point quotient for constraints without a closed form (angular rate):
-//   JT[k][r] = (F[k+1][r] - F[0][r]) / dx[k]      (_numdiff.py:709-711)
-__global__ void fd_quotient_kernel(const double *__restrict__ F, const double *__restrict__ dx,
-                                   int nvar, long long m, double *__restrict__ JT) {
-    const long long total = (long long)nvar * m;
-    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
-         idx += (long long)gridDim.x * blockDim.x) {
-        const long long k = idx / m, r = idx - k * m;
-        JT[idx] = __ddiv_rn(__dsub_rn(F[(k + 1) * m + r], F[r]), __ldg(dx + k));
-    }
-}
-
 }  // namespace
 
+// literal 2-point quotient for constraints without a closed form (angular rate), per sweep p:
+//   JT[p][k][r] = (F[p][k+1][r] - F[p][0][r]) / dx[p][k]      (_numdiff.py:709-711)
 static __global__ void fd_quotient_batched_kernel(const double *__restrict__ F, const double *__restrict__ dx,
                                            long long count, int nvar, long long m, double *__restrict__ JT) {
     const long long per = (long long)nvar * m, total = count * per;
@@ -628,14 +607,7 @@ extern "C" int bez_fd_quotient_batched(const double *d_F, const double *d_dx, in
 
 extern "C" int bez_fd_quotient(const double *d_F, const double *d_dx, int nvar, int64_t m,
                                double *d_JT, void *stream) {
-    BEZ_REQUIRE(d_F && d_dx && d_JT, "NULL argument");
-    BEZ_REQUIRE(nvar >= 0 && m >= 0, "negative size");
-    if (nvar == 0 || m == 0) return BEZ_OK;
-    long long blocks = ((long long)nvar * m + 255) / 256;
-    if (blocks > 148 * 32) blocks = 148 * 32;
-    fd_quotient_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(d_F, d_dx, nvar, m, d_JT);
-    BEZ_CUDA(cudaGetLastError());
-    return BEZ_OK;
+    return bez_fd_quotient_batched(d_F, d_dx, 1, nvar, m, d_JT, stream);
 }
 
 namespace {
@@ -664,27 +636,26 @@ int zero_rows(double *out, long long B, long long stride, long long off, long lo
     return BEZ_OK;
 }
 
-// Shared body of the single-point and batched separation Jacobians.  With one vehicle, the
-// leading N-1 pairs and ld = (N-1)*L, item (kk, uu) of the dense J^T lands at kk*ld + uu*L and
-// the tf rows at kdir*ld: a point's dense block is its sweep block byte for byte, nothing is left
-// to zero, and the dense request runs as a sweep (on the tensor path where L allows).  The
-// single-point entry keeps its kernel choice (dense_as_sweep = false) so its results stay those
-// of the dense kernel.  kdir >= 0 with d_dir == NULL: tf moves no control point, its rows are 0.
+// Shared body of the separation entries.  With one vehicle, the leading N-1 pairs and ld = (N-1)*L,
+// item (kk, uu) of the dense J^T lands at kk*ld + uu*L and the tf rows at kdir*ld: a point's dense
+// block is its sweep block byte for byte, nothing is left to zero, and the dense request runs as a
+// sweep (on the tensor path where L allows).  kdir >= 0 with d_dir == NULL: tf moves no control
+// point, its rows are 0.
 int jac_sep_impl(const bez_plan *plan, const double *d_cpts, long long B, int N, int numVeh, int ncols,
                  int offset, const double *d_dx, const double *d_dir, int kdir, long long npairs, int dense,
-                 double *d_out, int64_t ld, bool dense_as_sweep, cudaStream_t st) {
+                 double *d_out, int64_t ld, cudaStream_t st) {
     const long long L = plan->L;
     const long long nvarN = (long long)numVeh * plan->dim * ncols;
     const long long nvar = nvarN + (kdir >= 0 ? 1 : 0);
     const long long S = (plan->dim * (plan->n + 1) + 1) / 2 * 2;
     const long long ndir = kdir >= 0 ? npairs : 0;
     JacArgs A;
-    fill_common(plan, A, d_cpts, d_dir, d_dx, N, numVeh, ncols, offset, kdir, dense, d_out, ld);
-    A.scale = 0.5 * plan->dim;
-    A.B = B;
-    A.cstride = (long long)N * S;
-    A.dxstride = nvar;
-    if (dense && dense_as_sweep && numVeh == 1 && npairs == N - 1 && ld == npairs * L) A.dense = 0;
+    A.early_store = (bez_sq_elev_mma_flags() & kFlagEarlyFence) ? 1 : 0;
+    A.cpts = d_cpts; A.dir = d_dir; A.dx = d_dx; A.tfs = nullptr; A.PQ = plan->d_PQ; A.out = d_out;
+    A.B = B; A.cstride = (long long)N * S; A.dxstride = nvar; A.ld = ld;
+    A.N = N; A.numVeh = numVeh; A.L = plan->L; A.Lh = plan->Lh; A.LhPad = plan->LhPad;
+    A.ncols = ncols; A.offset = offset; A.kdir = kdir; A.tf = 1.0; A.scale = 0.5 * plan->dim;
+    A.dense = dense && !(numVeh == 1 && npairs == N - 1 && ld == npairs * L);
     A.ostride = A.dense ? nvar * ld : (nvarN * (N - 1) + ndir) * L;
     if (A.dense && (numVeh > 1 || npairs > N - 1 || ld > npairs * L)) {
         // rows of pairs without the variable's vehicle are never written
@@ -709,25 +680,23 @@ int jac_sep_impl(const bez_plan *plan, const double *d_cpts, long long B, int N,
     return BEZ_OK;
 }
 
-// Shared body of the speed Jacobians; d_tf [B] or NULL (the scalar tf).  kdir >= 0 with
-// d_dir == NULL: tf moves no control point, only the n/tf factor.
+// Shared body of the speed entries; d_tf [B] or NULL (the scalar tf).  One vehicle with ld = L:
+// J^T row kk is the sweep row of item kk, the tf row that of vehicle 0, so the dense request runs
+// as a sweep.  kdir >= 0 with d_dir == NULL: tf moves no control point, only the n/tf factor.
 int jac_speed_impl(const bez_plan *plan, const double *d_cpts, const double *d_tf, double tf, long long B,
                    int N, int numVeh, int ncols, int offset, double alpha, const double *d_dx, const double *d_dir,
-                   int kdir, int dense, double *d_out, int64_t ld, bool dense_as_sweep, cudaStream_t st) {
+                   int kdir, int dense, double *d_out, int64_t ld, cudaStream_t st) {
     const long long L = plan->L;
     const long long nvarN = (long long)numVeh * plan->dim * ncols;
     const long long nvar = nvarN + (kdir >= 0 ? 1 : 0);
     const long long S = (plan->dim * (plan->n + 1) + 1) / 2 * 2;
     JacArgs A;
-    fill_common(plan, A, d_cpts, d_dir, d_dx, N, numVeh, ncols, offset, kdir, dense, d_out, ld);
-    A.scale = alpha * 0.5 * plan->dim;
-    A.tf = tf;
-    A.tfs = d_tf;
-    A.B = B;
-    A.cstride = (long long)N * S;
-    A.dxstride = nvar;
-    // one vehicle with ld = L: J^T row kk is the sweep row of item kk, the tf row that of vehicle 0
-    if (dense && dense_as_sweep && numVeh == 1 && ld == L) A.dense = 0;
+    A.early_store = (bez_sq_elev_mma_flags() & kFlagEarlyFence) ? 1 : 0;
+    A.cpts = d_cpts; A.dir = d_dir; A.dx = d_dx; A.tfs = d_tf; A.PQ = plan->d_PQ; A.out = d_out;
+    A.B = B; A.cstride = (long long)N * S; A.dxstride = nvar; A.ld = ld;
+    A.N = N; A.numVeh = numVeh; A.L = plan->L; A.Lh = plan->Lh; A.LhPad = plan->LhPad;
+    A.ncols = ncols; A.offset = offset; A.kdir = kdir; A.tf = tf; A.scale = alpha * 0.5 * plan->dim;
+    A.dense = dense && !(numVeh == 1 && ld == L);
     A.ostride = A.dense ? nvar * ld : (nvarN + (kdir >= 0 ? numVeh : 0)) * L;
     if (A.dense && (numVeh > 1 || ld > (long long)numVeh * L))
         BEZ_CUDA(cudaMemsetAsync(d_out, 0, sizeof(double) * (size_t)(B * nvar * ld), st));
@@ -746,7 +715,19 @@ int jac_speed_impl(const bez_plan *plan, const double *d_cpts, const double *d_t
     return BEZ_OK;
 }
 
-int jac_degree_supported(const bez_plan *plan) {
+// Argument checks of the four entries, all before any CUDA call.  ptrs: every pointer the entry
+// needs is set; sep: the separation block (its leading npairs pairs), else the speed block.
+int jac_check(const bez_plan *plan, bool ptrs, bool sep, long long B, int N, int numVeh, int ncols, int offset,
+              int kdir, long long npairs, int dense, int64_t ld) {
+    BEZ_REQUIRE(plan && ptrs, "NULL argument");
+    BEZ_REQUIRE(B >= 0 && N >= (sep ? 2 : 1) && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0,
+                "bad sizes");
+    BEZ_REQUIRE(kdir < 0 || kdir == (long long)numVeh * plan->dim * ncols,
+                "kdir must be -1 or the index after the control-point variables");
+    const long long P = (long long)N * (N - 1) / 2, nObs = N - numVeh;
+    BEZ_REQUIRE(!sep || (npairs >= P - nObs * (nObs - 1) / 2 && npairs <= P),
+                "npairs must cover every pair that contains a vehicle and at most all pairs");
+    BEZ_REQUIRE(!dense || ld >= (sep ? npairs : numVeh) * (long long)plan->L, "ld smaller than the constraint block");
     if (plan->n < 1 || plan->n > BEZ_MAX_DEGREE_JAC || plan->dim < 1 || plan->dim > 3) {
         bez_set_error("degree %d, dimension %d: the Jacobian kernels cover n <= %d, dim <= 3", plan->n, plan->dim,
                       BEZ_MAX_DEGREE_JAC);
@@ -760,45 +741,30 @@ int jac_degree_supported(const bez_plan *plan) {
 extern "C" int bez_jac_sepsq_elev(const bez_plan *plan, const double *d_cpts, int N, int numVeh,
                                   int ncols, int offset, const double *d_dx, const double *d_dir,
                                   int kdir, int dense, double *d_out, int64_t ld, void *stream) {
-    BEZ_REQUIRE(plan && d_cpts && d_dx && d_out, "NULL argument");
-    BEZ_REQUIRE(N >= 2 && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0, "bad sizes");
-    BEZ_REQUIRE(kdir < 0 || d_dir, "direction rows are NULL");
-    const long long P = (long long)N * (N - 1) / 2;
-    BEZ_REQUIRE(!dense || ld >= P * plan->L, "ld smaller than the constraint block");
-    BEZ_ON_DEVICE(plan->device);
-    return jac_sep_impl(plan, d_cpts, 1, N, numVeh, ncols, offset, d_dx, d_dir, kdir, P, dense, d_out, ld, false,
-                        (cudaStream_t)stream);
+    return bez_jac_sepsq_elev_batched(plan, d_cpts, 1, N, numVeh, ncols, offset, d_dx, d_dir, kdir,
+                                      (int64_t)N * (N - 1) / 2, dense, d_out, ld, stream);
 }
 
 extern "C" int bez_jac_speed_sq_elev(const bez_plan *plan, const double *d_cpts, int N, int numVeh,
                                      int ncols, int offset, double tf, double alpha,
                                      const double *d_dx, const double *d_dir, int kdir, int dense,
                                      double *d_out, int64_t ld, void *stream) {
-    BEZ_REQUIRE(plan && d_cpts && d_dx && d_out, "NULL argument");
-    BEZ_REQUIRE(N >= 1 && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0, "bad sizes");
-    BEZ_REQUIRE(kdir < 0 || d_dir, "direction rows are NULL");
-    BEZ_REQUIRE(!dense || ld >= (long long)numVeh * plan->L, "ld smaller than the constraint block");
+    if (int rc = jac_check(plan, d_cpts && d_dx && d_out, false, 1, N, numVeh, ncols, offset, kdir, 0, dense, ld))
+        return rc;
     BEZ_ON_DEVICE(plan->device);
     return jac_speed_impl(plan, d_cpts, nullptr, tf, 1, N, numVeh, ncols, offset, alpha, d_dx, d_dir, kdir, dense,
-                          d_out, ld, false, (cudaStream_t)stream);
+                          d_out, ld, (cudaStream_t)stream);
 }
 
 extern "C" int bez_jac_sepsq_elev_batched(const bez_plan *plan, const double *d_cpts, int B, int N,
                                           int numVeh, int ncols, int offset, const double *d_dx,
                                           const double *d_dir, int kdir, int64_t npairs, int dense,
                                           double *d_out, int64_t ld, void *stream) {
-    BEZ_REQUIRE(plan && d_cpts && d_dx && d_out, "NULL argument");
-    BEZ_REQUIRE(B >= 0 && N >= 2 && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0, "bad sizes");
-    const long long nvarN = (long long)numVeh * plan->dim * ncols;
-    BEZ_REQUIRE(kdir < 0 || kdir == nvarN, "kdir must be -1 or the index after the control-point variables");
-    const long long P = (long long)N * (N - 1) / 2, nObs = N - numVeh;
-    BEZ_REQUIRE(npairs >= P - nObs * (nObs - 1) / 2 && npairs <= P,
-                "npairs must cover every pair that contains a vehicle and at most all pairs");
-    BEZ_REQUIRE(!dense || ld >= npairs * plan->L, "ld smaller than the constraint block");
-    if (int rc = jac_degree_supported(plan)) return rc;
+    if (int rc = jac_check(plan, d_cpts && d_dx && d_out, true, B, N, numVeh, ncols, offset, kdir, npairs, dense, ld))
+        return rc;
     if (B == 0) return BEZ_OK;
     BEZ_ON_DEVICE(plan->device);
-    return jac_sep_impl(plan, d_cpts, B, N, numVeh, ncols, offset, d_dx, d_dir, kdir, npairs, dense, d_out, ld, true,
+    return jac_sep_impl(plan, d_cpts, B, N, numVeh, ncols, offset, d_dx, d_dir, kdir, npairs, dense, d_out, ld,
                         (cudaStream_t)stream);
 }
 
@@ -806,14 +772,11 @@ extern "C" int bez_jac_speed_sq_elev_batched(const bez_plan *plan, const double 
                                              int B, int N, int numVeh, int ncols, int offset, double alpha,
                                              const double *d_dx, const double *d_dir, int kdir, int dense,
                                              double *d_out, int64_t ld, void *stream) {
-    BEZ_REQUIRE(plan && d_cpts && d_tf && d_dx && d_out, "NULL argument");
-    BEZ_REQUIRE(B >= 0 && N >= 1 && numVeh >= 1 && numVeh <= N && ncols >= 0 && offset >= 0, "bad sizes");
-    const long long nvarN = (long long)numVeh * plan->dim * ncols;
-    BEZ_REQUIRE(kdir < 0 || kdir == nvarN, "kdir must be -1 or the index after the control-point variables");
-    BEZ_REQUIRE(!dense || ld >= (long long)numVeh * plan->L, "ld smaller than the constraint block");
-    if (int rc = jac_degree_supported(plan)) return rc;
+    if (int rc = jac_check(plan, d_cpts && d_tf && d_dx && d_out, false, B, N, numVeh, ncols, offset, kdir, 0, dense,
+                           ld))
+        return rc;
     if (B == 0) return BEZ_OK;
     BEZ_ON_DEVICE(plan->device);
     return jac_speed_impl(plan, d_cpts, d_tf, 1.0, B, N, numVeh, ncols, offset, alpha, d_dx, d_dir, kdir, dense,
-                          d_out, ld, true, (cudaStream_t)stream);
+                          d_out, ld, (cudaStream_t)stream);
 }

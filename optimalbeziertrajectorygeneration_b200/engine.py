@@ -466,156 +466,6 @@ class ConstraintEngine:
             self._dir = D
         return self._dir
 
-    @_on_device
-    def jac_separation(self, x, elev, dense=True, out=None):
-        """FD Jacobian of the separation block at x (host vector).
-        dense: returns J^T as a device tensor [nvar, P*L]; else the sweep layout.
-        ``out``: preallocated destination of the right shape (sweep layout only)."""
-        plan = self.plan(elev)
-        x = np.asarray(x, dtype=np.float64)
-        _, dx = self.fd_steps(x)
-        d_dx = torch.as_tensor(dx, device=self.device)
-        cpts, _ = self.assemble(self.upload(x), elev)
-        dirs = self._direction_rows()
-        kdir = self.nvar - 1 if dirs is not None else -1
-        P, L = num_pairs(self.N), plan.L
-        nvarN = self.numVeh * self.dim * self.ncols
-        if dense:
-            out = torch.empty((self.nvar, P * L), dtype=F64, device=self.device)
-            if self.timeopt and dirs is None:
-                out[self.nvar - 1].zero_()          # tf does not move any control point
-            ld = P * L
-        else:
-            shape = (nvarN * (self.N - 1) + (P if kdir >= 0 else 0), L)
-            if out is None:
-                out = torch.empty(shape, dtype=F64, device=self.device)
-            elif tuple(out.shape) != shape or out.dtype != F64 or not out.is_contiguous():
-                raise ValueError("out must be a contiguous float64 tensor of shape %r" % (shape,))
-            ld = 0
-        _capi.call("bez_jac_sepsq_elev", plan.handle, _ptr(cpts), self.N, self.numVeh, self.ncols,
-                   self.offset, _ptr(d_dx), _ptr(dirs), kdir, int(dense), _ptr(out), ld, self._st())
-        return out
-
-    @_on_device
-    def jac_speed(self, x, elev, alpha, dense=True):
-        plan = self.plan(elev)
-        x = np.asarray(x, dtype=np.float64)
-        _, dx = self.fd_steps(x)
-        d_dx = torch.as_tensor(dx, device=self.device)
-        cpts, _ = self.assemble(self.upload(x), elev)
-        tf = float(x[-1]) if self.timeopt else self.tf_fixed
-        dirs = self._direction_rows()
-        if self.timeopt and dirs is None:
-            dirs = torch.zeros((self.N, self.row_stride), dtype=F64, device=self.device)
-        kdir = self.nvar - 1 if self.timeopt else -1
-        L = plan.L
-        nvarN = self.numVeh * self.dim * self.ncols
-        if dense:
-            out = torch.empty((self.nvar, self.numVeh * L), dtype=F64, device=self.device)
-            ld = self.numVeh * L
-        else:
-            out = torch.empty((nvarN + (self.numVeh if kdir >= 0 else 0), L), dtype=F64, device=self.device)
-            ld = 0
-        _capi.call("bez_jac_speed_sq_elev", plan.handle, _ptr(cpts), self.N, self.numVeh, self.ncols,
-                   self.offset, tf, float(alpha), _ptr(d_dx), _ptr(dirs), kdir, int(dense), _ptr(out),
-                   ld, self._st())
-        return out
-
-    def _batch_points(self, x):
-        """x [B, nvar] (host or device) -> (device x [B, nvar], SciPy's divisors [B, nvar])."""
-        if isinstance(x, torch.Tensor):
-            if x.dim() != 2 or int(x.shape[1]) != self.nvar:
-                raise ValueError("x must be [B, %d]" % self.nvar)
-            d_x = x.to(device=self.device, dtype=F64).contiguous()
-            return d_x, self._fd_steps_device(d_x)
-        x = np.asarray(x, dtype=np.float64)
-        if x.ndim != 2 or x.shape[1] != self.nvar:
-            raise ValueError("x must be [B, %d]" % self.nvar)
-        return self.upload(x), torch.as_tensor(self.fd_steps(x)[1], device=self.device)
-
-    def _batch_out(self, out, shape):
-        if out is None:
-            return torch.empty(shape, dtype=F64, device=self.device)
-        if tuple(out.shape) != shape or out.dtype != F64 or not out.is_contiguous():
-            raise ValueError("out must be a contiguous float64 tensor of shape %r" % (shape,))
-        self._check(out, shape, "out")
-        return out
-
-    @_on_device
-    def jac_separation_batched(self, x, elev, obst_sets=None, npairs=None, dense=True, out=None, base=None):
-        """SciPy's 2-point Jacobian of the separation block at B base points at once
-        (bez_jac_sepsq_elev_batched).  ``x`` [B, nvar], host or device; ``obst_sets``
-        [B, nObs, dim] (device): point b's own obstacles (problem batches); ``npairs``: the
-        leading pairs that get rows (default all; at least every pair with a vehicle).
-        dense: J^T [B, nvar, npairs*L]; else the sweep layout
-        [B, numVeh*dim*ncols*(N-1) + (npairs if time-optimal), L].
-        ``base``: (cpts, tf, dx) of assemble(x) already at hand (ProblemBatch.sweep)."""
-        plan = self.plan(elev)
-        P, L = num_pairs(self.N), plan.L
-        npairs = P if npairs is None else int(npairs)
-        if base is None:
-            d_x, d_dx = self._batch_points(x)
-            cpts, _ = self.assemble(d_x, elev, obst_sets=obst_sets, evals_per_set=1 if obst_sets is not None else 0)
-        else:
-            cpts, _, d_dx = base
-        B = int(cpts.shape[0])
-        kdir = self.nvar - 1 if self.timeopt else -1
-        nvarN = self.numVeh * self.dim * self.ncols
-        if dense:
-            shape = (B, self.nvar, npairs * L)
-        else:
-            shape = (B, nvarN * (self.N - 1) + (npairs if kdir >= 0 else 0), L)
-        out = self._batch_out(out, shape)
-        _capi.call("bez_jac_sepsq_elev_batched", plan.handle, _ptr(cpts), B, self.N, self.numVeh, self.ncols,
-                   self.offset, _ptr(d_dx), _ptr(self._direction_rows()), kdir, npairs, int(bool(dense)), _ptr(out),
-                   npairs * L if dense else 0, self._st())
-        return out
-
-    @_on_device
-    def jac_speed_batched(self, x, elev, alpha, dense=True, out=None, base=None):
-        """SciPy's 2-point Jacobian of the speed block alpha * (squared speed) + beta at B base
-        points at once (bez_jac_speed_sq_elev_batched); tf of each point from assemble.
-        dense: J^T [B, nvar, numVeh*L]; else [B, numVeh*dim*ncols + (numVeh if time-optimal), L].
-        ``base``: (cpts, tf, dx) of assemble(x) already at hand."""
-        plan = self.plan(elev)
-        L = plan.L
-        if base is None:
-            d_x, d_dx = self._batch_points(x)
-            cpts, tf = self.assemble(d_x, elev)
-        else:
-            cpts, tf, d_dx = base
-        B = int(cpts.shape[0])
-        kdir = self.nvar - 1 if self.timeopt else -1
-        nvarN = self.numVeh * self.dim * self.ncols
-        if dense:
-            shape = (B, self.nvar, self.numVeh * L)
-        else:
-            shape = (B, nvarN + (self.numVeh if kdir >= 0 else 0), L)
-        out = self._batch_out(out, shape)
-        _capi.call("bez_jac_speed_sq_elev_batched", plan.handle, _ptr(cpts), _ptr(tf), B, int(cpts.shape[1]),
-                   self.numVeh, self.ncols, self.offset, float(alpha), _ptr(d_dx), _ptr(self._direction_rows()),
-                   kdir, int(bool(dense)), _ptr(out), self.numVeh * L if dense else 0, self._st())
-        return out
-
-    @_on_device
-    def jac_angrate(self, x, elev, alpha, beta):
-        """Literal '2-point' FD Jacobian of the angular-rate block: base point and
-        all nvar perturbed points are evaluated in one batched launch (what SciPy
-        does serially with the reference), then differenced on the device.
-        Returns J^T [nvar, numVeh*(4m+1)]."""
-        x = np.asarray(x, dtype=np.float64)
-        h, dx = self.fd_steps(x)
-        X = np.repeat(x[None, :], self.nvar + 1, axis=0)
-        idx = np.arange(self.nvar)
-        X[idx + 1, idx] = x + h
-        cpts, tf = self.assemble(self.upload(X), elev)
-        F = self.angrate(cpts, tf, elev, alpha, beta).reshape(self.nvar + 1, -1)
-        m = int(F.shape[1])
-        d_dx = torch.as_tensor(dx, device=self.device)
-        JT = torch.empty((self.nvar, m), dtype=F64, device=self.device)
-        _capi.call("bez_fd_quotient", _ptr(F), _ptr(d_dx), self.nvar, m, _ptr(JT), self._st())
-        return JT
-
     @staticmethod
     def _fd_steps_device(d_x, abs_step=1.4901161193847656e-08):
         """dx of :meth:`fd_steps` for a device tensor (the same IEEE operations)."""
@@ -627,47 +477,143 @@ class ConstraintEngine:
         return (d_x + h) - d_x
 
     @_on_device
-    def jac_angrate_closed(self, x, elev, alpha, dense=True, out=None):
+    def _fd_base(self, x, elev, obst_sets=None):
+        """The base points of the closed-form Jacobians: ``x`` [nvar] or [B, nvar], host or device
+        -> (cpts [B, N, S], tf [B], SciPy's divisors dx [B, nvar], batched = x is 2-D), the tuple
+        their ``base=`` takes.  ``obst_sets`` [B, nObs, dim] (device): point b's own obstacles."""
+        on_device = isinstance(x, torch.Tensor)
+        x = x if on_device else np.asarray(x, dtype=np.float64)
+        if x.ndim not in (1, 2) or int(x.shape[-1]) != self.nvar:
+            raise ValueError("x must be [%d] or [B, %d]" % (self.nvar, self.nvar))
+        if on_device:
+            d_x = x.to(device=self.device, dtype=F64).reshape(-1, self.nvar).contiguous()
+            d_dx = self._fd_steps_device(d_x)
+        else:
+            x2 = np.atleast_2d(x)
+            d_x = self.upload(x2)
+            d_dx = torch.as_tensor(self.fd_steps(x2)[1], device=self.device)
+        cpts, tf = self.assemble(d_x, elev, obst_sets=obst_sets, evals_per_set=1 if obst_sets is not None else 0)
+        return cpts, tf, d_dx, x.ndim == 2
+
+    def _jac_out(self, out, shape, batched):
+        """Destination [B, rows, cols] of a closed-form Jacobian (``out`` or a new tensor), viewed
+        without the leading B for a 1-D x; a caller's ``out`` has x's rank."""
+        if out is None:
+            out = torch.empty(shape, dtype=F64, device=self.device)
+        else:
+            self._check(out, shape if batched else shape[1:], "out")
+        return out if batched else out.view(shape[1:])
+
+    @_on_device
+    def jac_separation(self, x, elev, dense=True, out=None, obst_sets=None, npairs=None, base=None):
+        """SciPy's 2-point Jacobian of the separation block in closed form (bez_jac_sepsq_elev_batched).
+        ``x`` [nvar] or [B, nvar], host or device; ``obst_sets`` [B, nObs, dim] (device): point b's
+        own obstacles (problem batches); ``npairs``: the leading pairs that get rows (default all;
+        at least every pair with a vehicle).
+        dense: J^T [B, nvar, npairs*L]; else the sweep layout
+        [B, numVeh*dim*ncols*(N-1) + (npairs if time-optimal), L]; without the leading B for 1-D x.
+        ``out``: the destination, in either layout and x's rank.
+        ``base``: :meth:`_fd_base` of x already at hand (ProblemBatch.sweep); x is then ignored."""
+        plan = self.plan(elev)
+        cpts, _, d_dx, batched = self._fd_base(x, elev, obst_sets) if base is None else base
+        B, L = int(cpts.shape[0]), plan.L
+        npairs = num_pairs(self.N) if npairs is None else int(npairs)
+        kdir = self.nvar - 1 if self.timeopt else -1
+        if dense:
+            shape = (B, self.nvar, npairs * L)
+        else:
+            shape = (B, self.numVeh * self.dim * self.ncols * (self.N - 1) + (npairs if self.timeopt else 0), L)
+        out = self._jac_out(out, shape, batched)
+        _capi.call("bez_jac_sepsq_elev_batched", plan.handle, _ptr(cpts), B, self.N, self.numVeh, self.ncols,
+                   self.offset, _ptr(d_dx), _ptr(self._direction_rows()), kdir, npairs, int(bool(dense)), _ptr(out),
+                   npairs * L if dense else 0, self._st())
+        return out
+
+    @_on_device
+    def jac_speed(self, x, elev, alpha, dense=True, out=None, base=None):
+        """SciPy's 2-point Jacobian of the speed block alpha * (squared speed) + beta in closed form
+        (bez_jac_speed_sq_elev_batched); tf of each point from assemble.  ``x``, ``out``, ``base``
+        as in :meth:`jac_separation`.
+        dense: J^T [B, nvar, numVeh*L]; else [B, numVeh*dim*ncols + (numVeh if time-optimal), L];
+        without the leading B for 1-D x."""
+        plan = self.plan(elev)
+        cpts, tf, d_dx, batched = self._fd_base(x, elev) if base is None else base
+        B, L = int(cpts.shape[0]), plan.L
+        kdir = self.nvar - 1 if self.timeopt else -1
+        if dense:
+            shape = (B, self.nvar, self.numVeh * L)
+        else:
+            shape = (B, self.numVeh * self.dim * self.ncols + (self.numVeh if self.timeopt else 0), L)
+        out = self._jac_out(out, shape, batched)
+        _capi.call("bez_jac_speed_sq_elev_batched", plan.handle, _ptr(cpts), _ptr(tf), B, int(cpts.shape[1]),
+                   self.numVeh, self.ncols, self.offset, float(alpha), _ptr(d_dx), _ptr(self._direction_rows()),
+                   kdir, int(bool(dense)), _ptr(out), self.numVeh * L if dense else 0, self._st())
+        return out
+
+    @_on_device
+    def fd_points(self, X):
+        """host X [B, nvar] -> device (Xp [B, nvar+1, nvar], dx [B, nvar]): the base point and the
+        nvar forward points of every row, h and dx as SciPy chooses them (:meth:`fd_steps`)."""
+        X = np.atleast_2d(np.asarray(X, dtype=np.float64))
+        B, n = X.shape[0], self.nvar
+        h, dx = self.fd_steps(X)
+        d_x, d_xh, d_dx = self.upload(np.concatenate((X, X + h, dx))).split(B)     # one pinned H2D
+        Xp = d_x[:, None, :].repeat(1, n + 1, 1)
+        Xp.view(B, -1)[:, n::n + 1] = d_xh          # forward point k+1 moves x_k: entry (k+1)*n + k
+        return Xp, d_dx
+
+    @_on_device
+    def fd_quotient(self, F, dx):
+        """SciPy's 2-point quotient of B sweeps (bez_fd_quotient_batched): F [B, nvar+1, m] holds
+        f at the base point and the nvar forward points of :meth:`fd_points`, dx [B, nvar] ->
+        J^T [B, nvar, m]."""
+        B, m = int(dx.shape[0]), int(F.shape[-1])
+        self._check(F, (B, self.nvar + 1, m), "F")
+        self._check(dx, (B, self.nvar), "dx")
+        JT = torch.empty((B, self.nvar, m), dtype=F64, device=self.device)
+        _capi.call("bez_fd_quotient_batched", _ptr(F), _ptr(dx), B, self.nvar, m, _ptr(JT), self._st())
+        return JT
+
+    @_on_device
+    def jac_angrate(self, x, elev, alpha, beta):
+        """Literal '2-point' FD Jacobian of the angular-rate block: base point and
+        all nvar perturbed points are evaluated in one batched launch (what SciPy
+        does serially with the reference), then differenced on the device.
+        Returns J^T [nvar, numVeh*(4m+1)]."""
+        Xp, dx = self.fd_points(x)
+        cpts, tf = self.assemble(Xp.view(-1, self.nvar), elev)
+        F = self.angrate(cpts, tf, elev, alpha, beta).view(1, self.nvar + 1, -1)
+        return self.fd_quotient(F, dx)[0]
+
+    @_on_device
+    def jac_angrate_closed(self, x, elev, alpha, dense=True, out=None, base=None):
         """Closed-form '2-point' Jacobian of the angular-rate block (bez_jac_angrate_sq): SciPy's
         quotient for the row alpha * (squared angular rate) + beta, without evaluating the
-        perturbed points.  ``x`` [nvar] or [B, nvar], host or device.
-        dense: J^T [nvar, numVeh*(4m+1)] ([B, nvar, ...] for 2-D x); else the sweep layout
-        [numVeh*2*ncols + (numVeh if time-optimal), 4m+1] (with a leading B for 2-D x).
+        perturbed points.  ``x``, ``out``, ``base`` as in :meth:`jac_separation` (the vehicle rows
+        of a base with obstacles serve as well).
+        dense: J^T [B, nvar, numVeh*(4m+1)]; else the sweep layout
+        [B, numVeh*2*ncols + (numVeh if time-optimal), 4m+1]; without the leading B for 1-D x.
         n + elev > 127 raises BezGpuError (jac_angrate covers those shapes)."""
         if self.dim != 2:
             raise ValueError('The input curve must be two dimensional,\n'
                              'instead it is {} dimensional'.format(self.dim))
         tabs = AngRateTables.get(self.n, elev, self.dev_index)
-        if isinstance(x, torch.Tensor):
-            batched = x.dim() == 2
-            d_x = x.to(device=self.device, dtype=F64).reshape(-1, self.nvar).contiguous()
-            d_dx = self._fd_steps_device(d_x)
-        else:
-            x = np.asarray(x, dtype=np.float64)
-            batched = x.ndim == 2
-            x2 = np.atleast_2d(x)
-            d_x = self.upload(x2)
-            d_dx = torch.as_tensor(self.fd_steps(x2)[1], device=self.device)
-        B = int(d_x.shape[0])
-        cpts, tf = self.assemble(d_x, elev)
-        dirs = self._direction_rows()
+        cpts, tf, d_dx, batched = self._fd_base(x, elev) if base is None else base
+        B = int(cpts.shape[0])
         kdir = self.nvar - 1 if self.timeopt else -1
         L4 = 4 * (self.n + int(elev)) + 1
         if dense:
             shape = (B, self.nvar, self.numVeh * L4)
         else:
-            shape = (B, self.numVeh * 2 * self.ncols + (self.numVeh if kdir >= 0 else 0), L4)
-        if out is None:
-            out = torch.empty(shape, dtype=F64, device=self.device)
-        else:
-            self._check(out, shape if batched else shape[1:], "out")
+            shape = (B, self.numVeh * 2 * self.ncols + (self.numVeh if self.timeopt else 0), L4)
+        out = self._jac_out(out, shape, batched)
         nscr = int(_capi.lib.bez_jac_angrate_scratch_doubles(B, self.numVeh, self.n, int(elev)))
         key = ("jac_angrate_scratch", nscr)
         scratch = getattr(self, "_scratch", {}).get(key)
         if scratch is None:
             scratch = torch.empty(max(nscr, 1), dtype=F64, device=self.device)
             self._scratch = {key: scratch}                 # one cached buffer per engine
-        _capi.call("bez_jac_angrate_sq", tabs.handle, _ptr(cpts), _ptr(tf), B, self.N, self.row_stride,
-                   self.numVeh, self.ncols, self.offset, self.nvar, _ptr(d_dx), _ptr(dirs), kdir,
+        _capi.call("bez_jac_angrate_sq", tabs.handle, _ptr(cpts), _ptr(tf), B, int(cpts.shape[1]), self.row_stride,
+                   self.numVeh, self.ncols, self.offset, self.nvar, _ptr(d_dx), _ptr(self._direction_rows()), kdir,
                    float(alpha), int(bool(dense)), _ptr(scratch), _ptr(out), shape[2], self._st())
-        return out if batched else out.view(shape[1:])
+        return out

@@ -302,17 +302,15 @@ class BezOptimization:
         warps); obstacle-obstacle rows are constants (zero rows)."""
         x = np.asarray(x, dtype=np.float64)
         eng = self._engine(with_obstacles=False)
-        h, dx = eng.fd_steps(x)
-        X = np.repeat(x[None, :], x.size + 1, axis=0)
-        idx = np.arange(x.size)
-        X[idx + 1, idx] = x + h
-        cpts, _ = eng.assemble(eng.upload(X), 0)
+        Xp, d_dx = eng.fd_points(x)
+        cpts, _ = eng.assemble(Xp.view(x.size + 1, x.size), 0)
         nrow = self.model['dim'] * (self.model['deg'] + 1)
         Y = eng.download(cpts[:, :, :nrow].contiguous(), key="spatial_y")
         Y = Y.reshape(x.size + 1, self.model['numVeh'] * self.model['dim'], self.model['deg'] + 1)
         rows, status = self._spatial_rows(Y)
         self._spatial_check(status)
         F = rows.reshape(x.size + 1, -1)
+        dx = eng.download(d_dx)[0]
         return ((F[1:] - F[0]) / dx[:, None]).T
 
     @property
@@ -488,16 +486,14 @@ class BezOptimization:
                 B = int(X.shape[0]) if isinstance(X, torch.Tensor) else np.atleast_2d(X).shape[0]
                 res['sep'] = torch.empty((B, eng.nvar, 0), dtype=torch.float64, device=eng.device)
             else:
-                res['sep'] = eng.jac_separation_batched(X, E, dense=True)
+                res['sep'] = eng.jac_separation(X, E, dense=True)
         if 'maxspeed' in which or 'minspeed' in which:
             eng = self._engine(with_obstacles=False)
-            d_x, d_dx = eng._batch_points(X)
-            cpts, tf = eng.assemble(d_x, E)
-            base = (cpts, tf, d_dx)
+            base = eng._fd_base(X, E)
             if 'maxspeed' in which:
-                res['maxspeed'] = eng.jac_speed_batched(None, E, -1.0, base=base)
+                res['maxspeed'] = eng.jac_speed(None, E, -1.0, base=base)
             if 'minspeed' in which:
-                res['minspeed'] = eng.jac_speed_batched(None, E, 1.0, base=base)
+                res['minspeed'] = eng.jac_speed(None, E, 1.0, base=base)
         return res
 
     @_on_model_device

@@ -1,5 +1,5 @@
 """Batched closed-form separation and speed Jacobians (bez_jac_sepsq_elev_batched,
-bez_jac_speed_sq_elev_batched, ConstraintEngine.jac_separation_batched / jac_speed_batched,
+bez_jac_speed_sq_elev_batched, ConstraintEngine.jac_separation / jac_speed with x [B, nvar],
 ProblemBatch "sep_closed" / "maxspeed_closed" / "minspeed_closed", BezOptimization.jacobian_batch).
 Judged like the single-point blocks: block-relative 1e-9 against the exactly rounded 2-point
 quotient of the oracle, and equal to the single-point closures problem by problem."""
@@ -139,8 +139,8 @@ def test_problem_batch_equals_single_example1(gopt, batch_mod, E):
 
 @pytest.mark.gpu
 def test_problem_batch_equals_single_c5(gopt, batch_mod):
-    """the C5 shape (n = 10, 16 obstacles, E = 100): the batch runs the one-vehicle dense block as
-    a tensor-path sweep, the single-point closure the dense kernel -- equal to rounding"""
+    """the C5 shape (n = 10, 16 obstacles, E = 100): batch and single-point closure both run the
+    one-vehicle dense block as a tensor-path sweep, so the results are identical"""
     E = 100
     probs, sets = _dubins_batch(3, nobs=16, deg=10, seed0=20)
     pb = batch_mod.ProblemBatch(_template(probs[0]), sets)
@@ -152,28 +152,37 @@ def test_problem_batch_equals_single_c5(gopt, batch_mod):
         for name in BLOCKS:
             J = res[name + "_closed"][1][i].cpu().numpy().T
             Js = single[name][:pb.npairs_x * L] if name == "sep" else single[name]
-            assert J.shape == Js.shape
-            scale = np.abs(Js).max()
-            assert np.abs(J - Js).max() <= 1e-13 * scale, (i, name)
+            assert np.array_equal(J, Js), (i, name)
 
 
 @pytest.mark.gpu
-def test_multi_start_equals_single(gopt):
-    """B = 5 different x of one 3-D swarm model without obstacles"""
-    E = 4
-    args, rng = _fixed_end(4, 3, 5, 'Euclidean', 9)
-    b = gopt.BezOptimization(**args)
-    eng = b._engine(True)
-    X = rng.normal(size=(5, b.nvar)) * 3
-    sep = eng.jac_separation_batched(X, E).cpu().numpy()
-    spd = eng.jac_speed_batched(X, E, -1.0).cpu().numpy()
-    for i in range(5):
-        assert np.array_equal(sep[i], eng.jac_separation(X[i], E).cpu().numpy()), i
-        assert np.array_equal(spd[i], eng.jac_speed(X[i], E, -1.0).cpu().numpy()), i
-    # device input: the same divisors and results
+def test_multi_start_points_equal_single_points(gopt):
+    """B = 5 different x of one swarm model without obstacles (3-D Euclidean; 2-D TimeOpt with the
+    angular-rate block): jac_*(X[i]) == jac_*(X)[i] bit for bit, both layouts, host and device input.
+    TimeOpt without Dubins ends: tf moves no control point (no direction rows, zero separation tf rows)"""
     import torch
-    assert torch.equal(eng.jac_separation_batched(torch.as_tensor(X, device=eng.device), E).cpu(),
-                       torch.as_tensor(sep))
+    E = 4
+    for goal, dim in (("Euclidean", 3), ("TimeOpt", 2)):
+        args, rng = _fixed_end(4, dim, 5, goal, 9)
+        b = gopt.BezOptimization(**args)
+        eng = b._engine(True)
+        X = rng.normal(size=(5, b.nvar)) * 3
+        if goal == "TimeOpt":
+            X[:, -1] = np.abs(X[:, -1]) + 8.0
+        jacs = {"sep": lambda x, dense: eng.jac_separation(x, E, dense=dense),
+                "speed": lambda x, dense: eng.jac_speed(x, E, -1.0, dense=dense)}
+        if dim == 2:
+            jacs["angrate"] = lambda x, dense: eng.jac_angrate_closed(x, E, -1.0, dense=dense)
+        d_X = torch.as_tensor(X, device=eng.device)
+        for name, jac in jacs.items():
+            for dense in (True, False):
+                what = (goal, name, dense)
+                JB = jac(X, dense).cpu().numpy()
+                assert JB.shape[0] == 5, what
+                assert np.array_equal(jac(d_X, dense).cpu().numpy(), JB), what
+                for i in range(5):
+                    assert np.array_equal(jac(X[i], dense).cpu().numpy(), JB[i]), what + (i,)
+                    assert np.array_equal(jac(d_X[i], dense).cpu().numpy(), JB[i]), what + (i,)
 
 
 # ---- 3. layouts --------------------------------------------------------------------------
@@ -197,7 +206,7 @@ def _sweep_to_dense_sep(sw, B, nvarN, N, numVeh, dim, ncols, L, npairs, kdir):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("V,dim,deg,E,B", [(9, 3, 10, 100, 3), (3, 2, 6, 60, 2), (4, 3, 5, 2, 3)])
-def test_sweep_rows_equal_dense_rows(gopt, V, dim, deg, E, B):
+def test_batched_sweep_rows_equal_dense_rows(gopt, V, dim, deg, E, B):
     """several vehicles: dense J^T on the dense kernel, the sweep layout on the tensor path where
     65 <= L <= 128 (V = 9, 3-D, n = 10, E = 100 runs the warp-specialised kernel: 1944 items per
     point, so tiles straddle variables, and the last tile of every point is partial)"""
@@ -208,15 +217,15 @@ def test_sweep_rows_equal_dense_rows(gopt, V, dim, deg, E, B):
     L = 2 * deg + E + 1
     P = V * (V - 1) // 2
     nvarN = eng.nvar
-    JT = eng.jac_separation_batched(X, E, dense=True).cpu().numpy()
-    sw = eng.jac_separation_batched(X, E, dense=False).cpu().numpy()
+    JT = eng.jac_separation(X, E, dense=True).cpu().numpy()
+    sw = eng.jac_separation(X, E, dense=False).cpu().numpy()
     assert sw.shape == (B, nvarN * (V - 1), L)
     D = _sweep_to_dense_sep(sw, B, nvarN, V, V, dim, eng.ncols, L, P, -1)
     scale = np.abs(JT).max()
     assert np.abs(D - JT).max() <= 1e-13 * scale
     assert np.array_equal(D == 0, JT == 0)
-    JS = eng.jac_speed_batched(X, E, 1.0, dense=True).cpu().numpy()
-    ss = eng.jac_speed_batched(X, E, 1.0, dense=False).cpu().numpy()
+    JS = eng.jac_speed(X, E, 1.0, dense=True).cpu().numpy()
+    ss = eng.jac_speed(X, E, 1.0, dense=False).cpu().numpy()
     assert ss.shape == (B, nvarN, L)
     v_of = np.arange(nvarN) // (dim * eng.ncols)
     for k in range(nvarN):
@@ -228,7 +237,7 @@ def test_sweep_rows_equal_dense_rows(gopt, V, dim, deg, E, B):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("nobs,deg,E", [(16, 10, 100), (5, 6, 3), (1, 10, 60)])
-def test_one_vehicle_dense_is_sweep(gopt, batch_mod, nobs, deg, E):
+def test_one_vehicle_dense_block_is_sweep_block(gopt, batch_mod, nobs, deg, E):
     """one vehicle, npairs = N-1: a point's dense J^T is its sweep block byte for byte"""
     import torch
     probs, sets = _dubins_batch(3, nobs=nobs, deg=deg, seed0=40)
@@ -236,17 +245,17 @@ def test_one_vehicle_dense_is_sweep(gopt, batch_mod, nobs, deg, E):
     eng = pb.eng
     X = _dubins_x(gopt, probs, 4)
     obst = pb.d_obst
-    d = eng.jac_separation_batched(X, E, obst_sets=obst, npairs=pb.npairs_x, dense=True)
-    s = eng.jac_separation_batched(X, E, obst_sets=obst, npairs=pb.npairs_x, dense=False)
+    d = eng.jac_separation(X, E, obst_sets=obst, npairs=pb.npairs_x, dense=True)
+    s = eng.jac_separation(X, E, obst_sets=obst, npairs=pb.npairs_x, dense=False)
     assert torch.equal(d.reshape(-1), s.reshape(-1))
-    d = eng.jac_speed_batched(X, E, -1.0, dense=True)
-    s = eng.jac_speed_batched(X, E, -1.0, dense=False)
+    d = eng.jac_speed(X, E, -1.0, dense=True)
+    s = eng.jac_speed(X, E, -1.0, dense=False)
     assert torch.equal(d.reshape(-1), s.reshape(-1))
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("V,obst", [(3, None), (1, [[0.5, -0.5]])])
-def test_timeopt_without_direction_rows(gopt, V, obst):
+def test_timeopt_tf_moves_no_control_point(gopt, V, obst):
     """fixed-end time-optimal: tf moves no control point -- its separation row is exactly zero,
     its speed row (the n/tf factor) is not; both match the oracle.  One vehicle and one obstacle:
     the dense block is the sweep block and only the tf row is zero-filled"""
@@ -262,7 +271,7 @@ def test_timeopt_without_direction_rows(gopt, V, obst):
     res = b.jacobian_batch(X, which=BLOCKS, elev=E)
     assert np.all(res["sep"][:, -1].cpu().numpy() == 0)
     assert np.all(np.abs(res["maxspeed"][:, -1].cpu().numpy()).max(axis=1) > 0)
-    sw = eng.jac_separation_batched(X, E, dense=False)
+    sw = eng.jac_separation(X, E, dense=False)
     nvarN, N = b.nvar - 1, eng.N
     P = N * (N - 1) // 2
     assert tuple(sw.shape) == (2, nvarN * (N - 1) + P, 2 * 5 + E + 1)
@@ -331,6 +340,14 @@ def test_errors_on_device(gopt):
     big = engine.Plan.get(13, 2, 0, dev.index)
     assert s(h=big.handle, ld=4 * 27) == -3
     assert v(h=big.handle, ld=27) == -3
+    # the single-point entries: B = 1 over all P = 10 pairs, the same checks
+    sep1, spd1 = _capi.lib.bez_jac_sepsq_elev, _capi.lib.bez_jac_speed_sq_elev
+    assert sep1(plan.handle, p, 5, 1, 3, 2, p, None, 6, 1, p, 10 * L, None) == 0
+    assert spd1(plan.handle, p, 5, 1, 3, 2, 8.0, -1.0, p, None, 6, 1, p, L, None) == 0
+    assert sep1(plan.handle, p, 5, 1, 3, 2, p, p, 2, 1, p, 10 * L, None) == -1
+    assert spd1(plan.handle, p, 5, 1, 3, 2, 8.0, -1.0, p, p, 2, 1, p, L, None) == -1
+    assert sep1(big.handle, p, 5, 1, 3, 2, p, p, 6, 1, p, 10 * 27, None) == -3
+    assert spd1(big.handle, p, 5, 1, 3, 2, 8.0, -1.0, p, p, 6, 1, p, 27, None) == -3
     torch.cuda.synchronize()
 
 
@@ -387,3 +404,22 @@ def test_argument_errors_without_gpu():
     assert v(h=ctypes.byref(big), ld=27) == -3
     # B = 0 is a no-op (still nothing touches the device)
     assert s(B=0) == 0 and v(B=0) == 0
+    # the single-point entries are B = 1 calls with the same checks (all P = 10 pairs)
+    sep1, spd1 = _capi.lib.bez_jac_sepsq_elev, _capi.lib.bez_jac_speed_sq_elev
+
+    def s1(h=ctypes.byref(plan), cpts=p, dx=p, out=p, kdir=6, ld=10 * 16):
+        return sep1(h, cpts, 5, 1, 3, 2, dx, p, kdir, 1, out, ld, None)
+
+    def v1(h=ctypes.byref(plan), cpts=p, dx=p, out=p, kdir=6, ld=16):
+        return spd1(h, cpts, 5, 1, 3, 2, 8.0, -1.0, dx, p, kdir, 1, out, ld, None)
+
+    for f in (s1, v1):
+        for bad in (dict(h=None), dict(cpts=None), dict(dx=None), dict(out=None)):
+            assert f(**bad) == -1, (f, bad)
+            assert "NULL" in _capi.last_error()
+        for kdir in (2, 7):
+            assert f(kdir=kdir) == -1 and "kdir" in _capi.last_error(), (f, kdir)
+    assert s1(ld=10 * 16 - 1) == -1 and "ld" in _capi.last_error()
+    assert v1(ld=15) == -1 and "ld" in _capi.last_error()
+    assert s1(h=ctypes.byref(big), ld=10 * 27) == -3
+    assert v1(h=ctypes.byref(big), ld=27) == -3

@@ -124,19 +124,19 @@ def w1(M, rounds, reps):
     def closed(block):
         def run():
             cpts, tf = eng.assemble(d_X, E, obst_sets=pb.d_obst, evals_per_set=1)
-            base = (cpts, tf, dx)
+            base = (cpts, tf, dx, True)
             if block == "sep":
                 eng.separation(cpts, E, m["maxSep"], pair_begin=0, npairs=pb.npairs_x)
-                eng.jac_separation_batched(None, E, npairs=pb.npairs_x, out=JC[block], base=base)
+                eng.jac_separation(None, E, npairs=pb.npairs_x, out=JC[block], base=base)
             else:
                 eng.speed(cpts, tf, E, -1.0, float(m["maxSpeed"]) ** 2)
-                eng.jac_speed_batched(None, E, -1.0, out=JC[block], base=base)
+                eng.jac_speed(None, E, -1.0, out=JC[block], base=base)
         return run
 
     cpts0, tf0 = eng.assemble(d_X, E, obst_sets=pb.d_obst, evals_per_set=1)
 
     def closed_jac_only():
-        eng.jac_separation_batched(None, E, npairs=pb.npairs_x, out=JC["sep"], base=(cpts0, tf0, dx))
+        eng.jac_separation(None, E, npairs=pb.npairs_x, out=JC["sep"], base=(cpts0, tf0, dx, True))
 
     blocks = ab({"sep_literal": literal("sep"), "sep_closed": closed("sep"), "sep_closed_jacobian_kernel_only":
                  closed_jac_only, "maxspeed_literal": literal("maxspeed"), "maxspeed_closed": closed("maxspeed")},
